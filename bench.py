@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W                 (N > 1: launched under torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W  the CPU arm (rank 0 only)
+    ... --dump-outputs DIR      also write the last timed step's placements (all ranks' queries) to DIR/*.npy
 
 Workload (SURVEY.md section 8d, config 5): synthetic 200 000-leaf Yule backbone, 5000-site nucleotide alignment
 evolved under JC69 with gaps, max-diameter clusters at 1.2 x 0.2, FM + MLSE, -f 0.2 -b 25 -V 0.001.  One "step" places
@@ -53,6 +54,9 @@ def parse(argv=None):
     ap.add_argument('--no-cli', action='store_true', help='skip the run_apples.py command-line measurement (cli_e2e)')
     ap.add_argument('--slot-cap', type=int, default=0, help='observed-list slots per query before a rerun (0 = library default)')
     ap.add_argument('--sub-batch', type=int, default=0, help='queries per dense/selection launch (0 = library default)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the placements of the last timed step as DIR/<name>.npy (float64), so that two builds can '
+                         'be compared output for output on the same seeded inputs')
     a = ap.parse_args(argv)
     prot = a.workload == 'protein'
     a.leaves = a.leaves or (4038 if prot else 200000)
@@ -208,6 +212,26 @@ def write_fasta(path, names, mat):
         f.write(out.tobytes())
 
 
+DUMP_BYTES_MAX = 64 << 20
+RESULT_NAMES = ('edge', 'error', 'distal', 'pendant', 'status')
+
+
+def dump_outputs(path, arrays):
+    """The five placement arrays of one step (edge, error, distal, pendant, status) -> <path>/<name>.npy in float64, which
+    holds the int32 edge and status exactly.  Above DUMP_BYTES_MAX in all, the same seeded sample of queries is written
+    every run, with the sampled query indices as query_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = [np.asarray(a) for a in arrays]
+    n = len(arrays[0])
+    idx = None
+    if 8 * n * len(arrays) > DUMP_BYTES_MAX:
+        k = (DUMP_BYTES_MAX - (64 << 10)) // (8 * (len(arrays) + 1))   # 64 KB left for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        np.save(os.path.join(path, 'query_index.npy'), idx.astype(np.float64))
+    for name, a in zip(RESULT_NAMES, arrays):
+        np.save(os.path.join(path, name + '.npy'), (a if idx is None else a[idx]).astype(np.float64))
+
+
 def cli_e2e(args, tree, host, q_bytes, device):
     """run_apples.py as a user runs it: reference FASTA + tree + cluster TSV + query FASTA on disk in, jplace on disk out.
     The files are written first (untimed); everything run_apples.main does is timed, stage by stage (its own timers)."""
@@ -285,9 +309,13 @@ def main():
         octx = cpu_context(args, tree, host)
         for s in range(args.warmup + args.steps):
             qs = q_host[s * n_sample:(s + 1) * n_sample]
-            r, dt, _ = cpu_baseline(octx, qs, threads)
+            r, dt, res = cpu_baseline(octx, qs, threads)
             if s >= args.warmup:
                 rates.append((r, dt))
+        if args.dump_outputs:
+            p = [x[0]['placements'][0]['p'][0] for x in res]
+            dump_outputs(args.dump_outputs, ([q[0] for q in p], [q[1] for q in p], [q[3] for q in p], [q[4] for q in p],
+                                             [x[1] for x in res]))
         tot_t = sum(dt for _, dt in rates)
         val = n_sample * len(rates) / tot_t
         line = {'impl': 'reference', 'metric': 'queries placed/sec', 'value': val, 'unit': 'queries/s',
@@ -369,6 +397,11 @@ def main():
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
     tm = pl.timings(reset=True)
+    last_step = None
+    if args.dump_outputs and rank == 0:
+        # taken here: the end-to-end steps below place the same queries again through the same context
+        last_step = ([t.cpu().numpy() for t in parallel.unpack_records(gathered[0])] if world > 1
+                     else pl.download_results())
     per_rank = None
     if world > 1:
         # every rank's own step time, dense-kernel time and the SM clock measured inside the dense kernel (clock64 /
@@ -641,6 +674,8 @@ def main():
                                           'under a fork pool of %d processes (%.1f s)' % (n_sample, n_ov, threads, dt),
                                 'parity_on_sample': '%d/%d identical edge; error, distal and pendant within 1e-9 '
                                                     '(%d overflow-rerun queries in the sample)' % (same, n_sample, n_ov)}
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, last_step)
     emit(line)
     if world > 1:
         dist.barrier()

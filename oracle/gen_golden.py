@@ -1,10 +1,11 @@
-"""Generates tests/golden/*.json by running the UNMODIFIED reference (/root/reference) in this container and
-asserts that oracle/apples_oracle.py reproduces it bit for bit.  TEST INFRASTRUCTURE.
+"""Generates tests/golden/*.json by running the UNMODIFIED reference (a checkout of the original APPLES, named by the
+environment variable APPLES_REFERENCE) and asserts that oracle/apples_oracle.py reproduces it bit for bit.  TEST
+INFRASTRUCTURE.
 
-Run:  python oracle/gen_golden.py        (build container only: /root/reference does not exist on the GPU box)
+Run:  APPLES_REFERENCE=<checkout of APPLES> python oracle/gen_golden.py
 
 What is the reference here and what is substituted:
-  * everything under /root/reference/apples is imported unmodified;
+  * everything under $APPLES_REFERENCE/apples is imported unmodified;
   * `treeswift` (absent dependency) is oracle/treeswift_shim;
   * `TreeCluster.py` (absent dependency) cannot run, so the cluster TSV is produced by apples_b200.treecluster and
     fed to the reference's own parsing + PoolRepresentativeWorker code (Reference.py:94-107), i.e. a
@@ -16,7 +17,7 @@ script reads them, it does not regenerate them, so the vectors stay pinned whate
 apples_b200.treecluster become.  `--regen-inputs` rebuilds the synthetic inputs (syn300*, prot_*) and the cluster TSVs
 from their seeds first (only when a fixture is to be replaced on purpose).  `--check` writes nothing: it regenerates
 every vector into a scratch directory and fails if any committed tests/golden/*.json would change
-(tests/test_oracle_golden.py::test_golden_recipe_reproduces_committed_vectors runs it where /root/reference exists).
+(tests/test_oracle_golden.py::test_golden_recipe_reproduces_committed_vectors runs it where APPLES_REFERENCE is set).
 """
 import gzip
 import itertools
@@ -32,8 +33,9 @@ import numpy as np
 warnings.filterwarnings('ignore')
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.abspath(os.path.join(HERE, '..'))
+REFERENCE = os.environ.get('APPLES_REFERENCE', '')
 sys.path.insert(0, os.path.join(HERE, 'treeswift_shim'))
-sys.path.insert(0, '/root/reference')
+sys.path.insert(0, REFERENCE)
 sys.path.insert(0, ROOT)
 
 from apples.PoolQueryWorker import PoolQueryWorker  # noqa: E402
@@ -56,7 +58,7 @@ from apples_b200.tree import BackboneTree  # noqa: E402
 GOLD = os.path.join(ROOT, 'tests', 'golden')
 DATA = os.path.join(GOLD, 'data')
 OUT = GOLD   # --check redirects the vectors to a scratch directory
-REF_DATA = '/root/reference/data'
+REF_DATA = os.path.join(REFERENCE, 'data')
 ALGS = {'FM': FM, 'OLS': OLS, 'BME': BME, 'BE': BE}
 
 

@@ -104,12 +104,13 @@ def test_alignment_and_matrix_agree():
 def test_golden_recipe_reproduces_committed_vectors():
     """oracle/gen_golden.py --check: the committed recipe, fed with the committed input fixtures and run against the
     UNMODIFIED reference, regenerates every tests/golden/*.json byte for byte (and asserts oracle == reference bit for
-    bit on the way).  Catches drift between recipe, fixtures and oracle; runs only where /root/reference exists."""
+    bit on the way).  Catches drift between recipe, fixtures and oracle; runs only where the environment variable
+    APPLES_REFERENCE names a checkout of the original APPLES (its apples/ package and data/ directory)."""
     import os
     import subprocess
     import sys
-    if not os.path.isdir('/root/reference/apples'):
-        pytest.skip('/root/reference is not present on this box')
+    if not os.path.isdir(os.path.join(os.environ.get('APPLES_REFERENCE', ''), 'apples')):
+        pytest.skip('needs the original APPLES sources: set APPLES_REFERENCE to a checkout of them')
     r = subprocess.run([sys.executable, os.path.join(util.ROOT, 'oracle', 'gen_golden.py'), '--check'],
                        stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:]
