@@ -25,7 +25,7 @@ SYMBOLS = [
     'apples_words_per_row', 'apples_aa_row_bytes', 'apples_device_count', 'apples_ctx_create', 'apples_ctx_destroy', 'apples_last_error',
     'apples_ctx_stream', 'apples_ctx_set_limits', 'apples_ctx_set_dense_mode', 'apples_set_tree', 'apples_set_reference', 'apples_set_matrix_columns', 'apples_place_batch',
     'apples_place_batch_matrix', 'apples_set_reference_bytes', 'apples_place_batch_bytes', 'apples_queries_upload', 'apples_place_resident', 'apples_results_download', 'apples_results_to_device',
-    'apples_distance_counts', 'apples_observed_sets', 'apples_edge_solutions', 'apples_get_timings', 'apples_last_counts',
+    'apples_distance_counts', 'apples_count_keys', 'apples_observed_sets', 'apples_edge_solutions', 'apples_get_timings', 'apples_last_counts',
     'apples_fasta_open', 'apples_fasta_close', 'apples_fasta_count', 'apples_fasta_max_len', 'apples_fasta_stride',
     'apples_fasta_uniform', 'apples_fasta_pinned', 'apples_fasta_matrix', 'apples_fasta_lengths', 'apples_fasta_names',
     'apples_fasta_name_offsets', 'apples_jplace_write',
@@ -81,6 +81,7 @@ def load():
     lib.apples_results_download.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_results_to_device.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_distance_counts.argtypes = [vp, i64, vp, dbl, vp, vp, vp]
+    lib.apples_count_keys.argtypes = [vp, i64, vp, C.POINTER(Params), C.POINTER(i32), vp]
     lib.apples_observed_sets.argtypes = [vp, i64, vp, vp, vp, C.POINTER(Params), i32, vp, vp, vp]
     lib.apples_edge_solutions.argtypes = [vp, vp, vp, i32, C.POINTER(Params), vp, vp, vp, vp]
     lib.apples_get_timings.argtypes = [vp, vp, C.c_int, C.c_int]

@@ -310,6 +310,10 @@ struct BatchIO {
     // parity exports
     int obs_cap = 0; int32_t* obs_count = nullptr; int32_t* obs_node = nullptr; double* obs_dist = nullptr;
     bool stop_after_select = false;
+    // count-keys export: every sub-batch's [nb][n_rep] block of the key matrix is copied to h_keys and the batch stops
+    // after the count stage (no selection, no placement)
+    void* h_keys = nullptr;
+    bool stop_after_count = false;
     double* dbg_x1 = nullptr; double* dbg_x2 = nullptr; double* dbg_err = nullptr; uint8_t* dbg_valid = nullptr;
 };
 
@@ -538,6 +542,13 @@ int run_macro(apples_ctx* ctx, int64_t base0, int n, const BatchIO& io, const ap
             ctx->n_pairs += (double)nb * ctx->n_rep;
         }
         CK(cudaGetLastError());
+        if (io.stop_after_count) {
+            // the rows of this sub-batch, without the padding columns of the key matrix
+            const size_t row = (size_t)n_units * key_bytes;
+            CK(cudaMemcpy2DAsync((char*)io.h_keys + (size_t)(base0 + a.q_begin) * row, row, slow ? kw : ctx->keys.p,
+                                 (size_t)ldk * key_bytes, row, nb, cudaMemcpyDeviceToHost, cur));
+            return 0;
+        }
         a.n = nb;
         a.q_nuc = (const uint32_t*)d_q;
         a.q_aa = (const uint8_t*)d_q;
@@ -629,6 +640,11 @@ int run_macro(apples_ctx* ctx, int64_t base0, int n, const BatchIO& io, const ap
         sa.q_begin = sb0;
         if (distances_and_select(d_q, nb, sa, false, slow_ctx, (const uint8_t*)ctx->q_bytes_p.p, ctx->keys.p)) return -1;
         if (used[buf]) CK(cudaEventRecord(ctx->ev_free[buf], s));
+    }
+    if (io.stop_after_count) {
+        CK(cudaStreamSynchronize(s));
+        collect_spans(ctx);
+        return 0;
     }
 
     // launch classes of the placeable queries, sorted on the device (counts: 5 ints at offset 0, stats: 4 u64 at offset 32)
@@ -1545,6 +1561,19 @@ int apples_distance_counts(apples_ctx* ctx, int64_t nq, const void* packed_queri
     if (e != cudaSuccess) rc = fail(ctx, "apples_distance_counts: %s", cudaGetErrorString(e));
     cleanup();
     return rc;
+}
+
+int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, const apples_params* params,
+                      int32_t* key_kind, void* keys) {
+    if (!ctx) return -1;
+    if (ctx->kind < 0) return fail(ctx, "apples_set_reference has not been called");
+    if (nq <= 0 || !packed_queries || !key_kind || !keys) return fail(ctx, "apples_count_keys: bad arguments");
+    *key_kind = ctx->kind == APPLES_AA ? 2 : (ctx->nuc_slow ? 1 : 0);
+    BatchIO io;
+    io.h_queries = packed_queries;
+    io.h_keys = keys;
+    io.stop_after_count = true;
+    return run_batch(ctx, nq, io, params);
 }
 
 int apples_observed_sets(apples_ctx* ctx, int64_t nq, const void* packed_queries, const double* rows,

@@ -46,6 +46,7 @@ class GpuPlacer:
         self.reference = None
         self.kind = None
         self.L = None
+        self.n_rep = None
         self.ref_names = None
         self.matrix_tags = None
         if reference is not None:
@@ -84,18 +85,24 @@ class GpuPlacer:
         """on_device: ship the raw alignment bytes and let the device pack them and build the consensus
         representatives (SURVEY.md section 8 f1/f2); otherwise pack / build on the host with numpy."""
         if on_device and hasattr(reference, 'device_arrays_bytes'):
-            d = reference.device_arrays_bytes(self.name_to_node)
-            self.kind, self.L, self.ref_names = d['kind'], int(d['L']), d['ref_names']
-            rb, rn, go, gm = d['ref_bytes'], d['ref_node'], d['group_offsets'], d['group_members']
-            if not (rb.dtype == np.uint8 and rb.ndim == 2 and rb.strides[1] == 1 and rb.strides[0] >= rb.shape[1]):
-                rb = np.ascontiguousarray(rb, dtype=np.uint8)
-            # rows may be padded (the native reader's matrix): the stride is passed on, no gigabyte-sized copy
-            self._check(self.lib.apples_set_reference_bytes(self.h, self.kind, self.L, rb.shape[0], rb.ctypes.data,
-                                                            rb.strides[0] if rb.shape[0] else self.L, _lib.ptr(rn),
-                                                            len(go) - 1, _lib.ptr(go), _lib.ptr(gm)))
+            self.set_reference_bytes(**reference.device_arrays_bytes(self.name_to_node))
         else:
             self.set_reference_arrays(**reference.device_arrays(self.name_to_node))
         self.reference = reference
+
+    def set_reference_bytes(self, kind, L, ref_names, ref_bytes, ref_node, group_offsets, group_members):
+        """Alignment bytes of the references; the device packs them and builds the consensus representatives."""
+        self.kind, self.L, self.ref_names, self.n_rep = kind, int(L), ref_names, len(group_offsets) - 1
+        rb = ref_bytes
+        if not (rb.dtype == np.uint8 and rb.ndim == 2 and rb.strides[1] == 1 and rb.strides[0] >= rb.shape[1]):
+            rb = np.ascontiguousarray(rb, dtype=np.uint8)
+        go = np.ascontiguousarray(group_offsets, dtype=np.int32)
+        gm = np.ascontiguousarray(group_members, dtype=np.int32)
+        rn = np.ascontiguousarray(ref_node, dtype=np.int32)
+        # rows may be padded (the native reader's matrix): the stride is passed on, no gigabyte-sized copy
+        self._check(self.lib.apples_set_reference_bytes(self.h, kind, self.L, rb.shape[0], rb.ctypes.data,
+                                                        rb.strides[0] if rb.shape[0] else self.L, _lib.ptr(rn),
+                                                        self.n_rep, _lib.ptr(go), _lib.ptr(gm)))
 
     def set_reference_arrays(self, kind, L, ref_names, packed_refs, ref_node, packed_reps, group_offsets, group_members):
         self.kind, self.L, self.ref_names = kind, int(L), ref_names
@@ -103,6 +110,7 @@ class GpuPlacer:
                       np.ascontiguousarray(packed_reps), np.ascontiguousarray(group_offsets, dtype=np.int32),
                       np.ascontiguousarray(group_members, dtype=np.int32))
         pr, rn, pp, go, gm = self._keep
+        self.n_rep = pp.shape[0]
         self._check(self.lib.apples_set_reference(self.h, kind, int(L), pr.shape[0], _lib.ptr(pr), _lib.ptr(rn),
                                                   pp.shape[0], _lib.ptr(pp), _lib.ptr(go), _lib.ptr(gm)))
         self._keep = None
@@ -212,6 +220,18 @@ class GpuPlacer:
         self._check(self.lib.apples_distance_counts(self.h, nq, _lib.ptr(packed), float(overlap_frac), _lib.ptr(mism),
                                                     _lib.ptr(valid), _lib.ptr(dist)))
         return mism, valid, dist
+
+    def count_keys(self, packed, params):
+        """Query x representative keys of the hot path's count stage (apples_count_keys): ([nq, n_rep] array, kind) with
+        kind 0 = uint32 mismatch | valid << 16, 1 = uint64 mismatch | valid << 32 (byte mode), 2 = float64 scoredist."""
+        packed = np.ascontiguousarray(packed)
+        nq = int(packed.shape[0])
+        raw = np.zeros(nq * self.n_rep, np.uint64)
+        kind = _lib.C.c_int32(-1)
+        self._check(self.lib.apples_count_keys(self.h, nq, _lib.ptr(packed), _lib.C.byref(params), _lib.C.byref(kind),
+                                               _lib.ptr(raw)))
+        dtype = {0: np.uint32, 1: np.uint64, 2: np.float64}[kind.value]
+        return raw.view(dtype)[:nq * self.n_rep].reshape(nq, self.n_rep), kind.value
 
     def observed_sets(self, params, packed=None, rows=None, self_node=None, cap=4096):
         src = packed if packed is not None else rows

@@ -145,6 +145,16 @@ int apples_results_to_device(apples_ctx* ctx, void* edge, void* error, void* dis
 int apples_distance_counts(apples_ctx* ctx, int64_t nq, const void* packed_queries, double overlap_frac,
                            uint32_t* mism, uint32_t* valid, double* dist);
 
+/* kernel (a) as the hot path runs it: the query x REPRESENTATIVE keys of nq packed queries, straight from the count stage
+ * of apples_place_batch (same kernels, kernel choice, sub-batches and key-matrix layout; the batch stops before the
+ * selection).  keys is [nq][n_rep] (padding columns dropped); *key_kind tells what it holds:
+ *   0  uint32  mismatch | valid << 16   (tensor-core or integer-pipe kernel)
+ *   1  uint64  mismatch | valid << 32   (byte-compare fallback: L > 65 535 or bytes other than A,C,G,T,- in the reference)
+ *   2  double  scoredist with params->overlap_frac (APPLES_AA)
+ * The caller sizes keys for 8 bytes per entry unless it knows the context's kind. */
+int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, const apples_params* params,
+                      int32_t* key_kind, void* keys);
+
 /* kernel (c): the observed set of each query as the reference would hold it after PoolQueryWorker.py:40-70 (self
  * entry removed), sorted by node id; count[q] may exceed cap (then only cap entries are written).
  * Exactly one of packed_queries / rows is non-NULL. */
