@@ -18,6 +18,7 @@ STATUS_CODE_MASK = 0xff
 PLACED, ZERO_DIST_LEAF, TOO_FEW_DISTANCES, PLACED_MISPLACEMENT_FLAG = 0, 1, 2, 3
 FLAG_PENDANT_INT0 = 0x100
 FLAG_DEGENERATE = 0x200
+MAX_KEEP = 16            # APPLES_MAX_KEEP: ranked records per query (apples_set_alternatives)
 NEWICK_UNSUPPORTED = 1   # apples_newick_*: text outside the native parser's language, use the Python twin
 
 # every symbol the header declares (tests/test_cabi.py checks the library exports exactly these)
@@ -25,10 +26,10 @@ SYMBOLS = [
     'apples_words_per_row', 'apples_aa_row_bytes', 'apples_device_count', 'apples_ctx_create', 'apples_ctx_destroy', 'apples_last_error',
     'apples_ctx_stream', 'apples_ctx_set_limits', 'apples_ctx_set_dense_mode', 'apples_set_tree', 'apples_set_reference', 'apples_set_matrix_columns', 'apples_place_batch',
     'apples_place_batch_matrix', 'apples_set_reference_bytes', 'apples_place_batch_bytes', 'apples_queries_upload', 'apples_place_resident', 'apples_results_download', 'apples_results_to_device',
-    'apples_distance_counts', 'apples_count_keys', 'apples_observed_sets', 'apples_edge_solutions', 'apples_get_timings', 'apples_last_counts',
+    'apples_set_alternatives', 'apples_distance_counts', 'apples_count_keys', 'apples_observed_sets', 'apples_edge_solutions', 'apples_get_timings', 'apples_last_counts',
     'apples_fasta_open', 'apples_fasta_close', 'apples_fasta_count', 'apples_fasta_max_len', 'apples_fasta_stride',
     'apples_fasta_uniform', 'apples_fasta_pinned', 'apples_fasta_matrix', 'apples_fasta_lengths', 'apples_fasta_names',
-    'apples_fasta_name_offsets', 'apples_jplace_write',
+    'apples_fasta_name_offsets', 'apples_jplace_write', 'apples_jplace_write_k',
     'apples_newick_parse', 'apples_newick_free', 'apples_newick_nodes', 'apples_newick_rooted', 'apples_newick_parent',
     'apples_newick_level', 'apples_newick_first', 'apples_newick_edge_length', 'apples_newick_has_length',
     'apples_newick_has_label', 'apples_newick_labels', 'apples_newick_label_offsets', 'apples_newick_extended',
@@ -78,6 +79,7 @@ def load():
     lib.apples_place_batch_bytes.argtypes = [vp, i64, vp, i64, vp, C.POINTER(Params), vp, vp, vp, vp, vp]
     lib.apples_queries_upload.argtypes = [vp, i64, vp, vp]
     lib.apples_place_resident.argtypes = [vp, C.POINTER(Params)]
+    lib.apples_set_alternatives.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
     lib.apples_results_download.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_results_to_device.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_distance_counts.argtypes = [vp, i64, vp, dbl, vp, vp, vp]
@@ -100,6 +102,8 @@ def load():
         getattr(lib, 'apples_fasta_' + fn).restype = vp
     lib.apples_jplace_write.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, i64, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int,
                                         C.c_int, C.POINTER(i64), C.c_char_p, C.c_int]
+    lib.apples_jplace_write_k.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, i64, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int,
+                                          i32, vp, vp, vp, vp, vp, vp, C.c_int, C.POINTER(i64), C.c_char_p, C.c_int]
     lib.apples_newick_parse.argtypes = [vp, i64, C.POINTER(vp), C.c_char_p, C.c_int]
     lib.apples_newick_free.argtypes = [vp]
     lib.apples_newick_free.restype = None

@@ -31,6 +31,17 @@ struct TimedSpan {
     cudaEvent_t a, b;
 };
 
+// host buffers of the ranked records (apples_set_alternatives); keep 1: none
+struct AltOut {
+    int keep = 1;
+    int32_t* count = nullptr;
+    int32_t* edge = nullptr;
+    double* error = nullptr;
+    double* distal = nullptr;
+    double* pendant = nullptr;
+    uint8_t* int0 = nullptr;
+};
+
 }  // namespace
 
 struct apples_ctx {
@@ -75,6 +86,8 @@ struct apples_ctx {
     double dense_mhz = 0.0;  // effective SM clock of the last dense launch (clock64 / globaltimer of CTA 0)
     DevBuf obs_node2, obs_dist2, qlist, pl_lists, bin_counts, bin_lists, rec_off, stack_off, recs, stacks;
     DevBuf o_edge, o_err, o_distal, o_pendant, o_status;
+    DevBuf o_alt_count, o_alt_edge, o_alt_err, o_alt_distal, o_alt_pendant, o_alt_int0;
+    AltOut alt;   // registered by apples_set_alternatives, taken by the next apples_place_batch* call
     DevBuf dbg_x1, dbg_x2, dbg_err, dbg_valid;
     // resident queries
     DevBuf res_q, res_self;
@@ -362,6 +375,7 @@ struct BatchIO {
     void* h_keys = nullptr;
     bool stop_after_count = false;
     double* dbg_x1 = nullptr; double* dbg_x2 = nullptr; double* dbg_err = nullptr; uint8_t* dbg_valid = nullptr;
+    AltOut alt;   // ranked records [nq][alt.keep] when alt.keep > 1 (host output only)
 };
 
 int check_params(apples_ctx* ctx, const apples_params* p) {
@@ -532,6 +546,13 @@ struct MacroBatch {
             ensure(ctx, ctx->o_distal, (size_t)n * 8) || ensure(ctx, ctx->o_pendant, (size_t)n * 8) ||
             ensure(ctx, ctx->o_status, (size_t)n * 4))
             return -1;
+        if (io.alt.keep > 1) {
+            const size_t nk = (size_t)n * io.alt.keep;
+            if (ensure(ctx, ctx->o_alt_count, (size_t)n * 4) || ensure(ctx, ctx->o_alt_edge, nk * 4) ||
+                ensure(ctx, ctx->o_alt_err, nk * 8) || ensure(ctx, ctx->o_alt_distal, nk * 8) ||
+                ensure(ctx, ctx->o_alt_pendant, nk * 8) || ensure(ctx, ctx->o_alt_int0, nk))
+                return -1;
+        }
         if (ensure(ctx, ctx->rec_off, (size_t)(n + 1) * 8) || ensure(ctx, ctx->stack_off, (size_t)(n + 1) * 8) ||
             ensure(ctx, ctx->qlist, (size_t)std::max(n, 1) * 4) || ensure(ctx, ctx->pl_lists, (size_t)std::max(n, 1) * 8))
             return -1;
@@ -622,6 +643,15 @@ struct MacroBatch {
         pa.out_distal = (double*)ctx->o_distal.p;
         pa.out_pendant = (double*)ctx->o_pendant.p;
         pa.out_status = (int*)ctx->o_status.p;
+        pa.keep = io.alt.keep;
+        if (io.alt.keep > 1) {
+            pa.alt_count = (int*)ctx->o_alt_count.p;
+            pa.alt_edge = (int*)ctx->o_alt_edge.p;
+            pa.alt_error = (double*)ctx->o_alt_err.p;
+            pa.alt_distal = (double*)ctx->o_alt_distal.p;
+            pa.alt_pendant = (double*)ctx->o_alt_pendant.p;
+            pa.alt_int0 = (unsigned char*)ctx->o_alt_int0.p;
+        }
         pa.dbg_query = dbg ? 0 : -1;
         pa.dbg_x1 = dbg ? (double*)ctx->dbg_x1.p : nullptr;
         pa.dbg_x2 = (double*)ctx->dbg_x2.p;
@@ -1137,6 +1167,16 @@ struct MacroBatch {
         CK(cudaMemcpyAsync(io.distal + base0, ctx->o_distal.p, (size_t)n * 8, kd, s));
         CK(cudaMemcpyAsync(io.pendant + base0, ctx->o_pendant.p, (size_t)n * 8, kd, s));
         CK(cudaMemcpyAsync(io.status + base0, ctx->o_status.p, (size_t)n * 4, kd, s));
+        const AltOut& al = io.alt;
+        if (al.keep > 1) {
+            const size_t o = (size_t)base0 * al.keep, nk = (size_t)n * al.keep;
+            CK(cudaMemcpyAsync(al.count + base0, ctx->o_alt_count.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(al.edge + o, ctx->o_alt_edge.p, nk * 4, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(al.error + o, ctx->o_alt_err.p, nk * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(al.distal + o, ctx->o_alt_distal.p, nk * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(al.pendant + o, ctx->o_alt_pendant.p, nk * 8, cudaMemcpyDeviceToHost, s));
+            CK(cudaMemcpyAsync(al.int0 + o, ctx->o_alt_int0.p, nk, cudaMemcpyDeviceToHost, s));
+        }
         return 0;
     }
 
@@ -1162,6 +1202,13 @@ struct MacroBatch {
         return 0;
     }
 };
+
+// the registration of apples_set_alternatives, cleared: it serves one apples_place_batch* call
+AltOut take_alternatives(apples_ctx* ctx) {
+    const AltOut a = ctx->alt;
+    ctx->alt = AltOut{};
+    return a;
+}
 
 int run_macro(apples_ctx* ctx, int64_t base0, int n, const BatchIO& io, const apples_params* prm) {
     return MacroBatch(ctx, base0, n, io, prm).run();
@@ -1339,16 +1386,37 @@ int apples_set_matrix_columns(apples_ctx* ctx, int32_t n_cols, const int32_t* co
     return 0;
 }
 
+int apples_set_alternatives(apples_ctx* ctx, int32_t keep, int32_t* count, int32_t* edge, double* error, double* distal,
+                            double* pendant, uint8_t* pendant_int0) {
+    if (!ctx) return -1;
+    ctx->alt = AltOut{};
+    if (keep < 1 || keep > APPLES_MAX_KEEP)
+        return fail(ctx, "apples_set_alternatives: keep = %d is outside [1, %d]", keep, APPLES_MAX_KEEP);
+    const int given = !!count + !!edge + !!error + !!distal + !!pendant + !!pendant_int0;
+    if (keep == 1 || given == 0) return 0;
+    if (given != 6) return fail(ctx, "apples_set_alternatives: pass all six buffers or none");
+    ctx->alt.keep = keep;
+    ctx->alt.count = count;
+    ctx->alt.edge = edge;
+    ctx->alt.error = error;
+    ctx->alt.distal = distal;
+    ctx->alt.pendant = pendant;
+    ctx->alt.int0 = pendant_int0;
+    return 0;
+}
+
 int apples_place_batch(apples_ctx* ctx, int64_t nq, const void* packed_queries, const int32_t* self_node,
                        const apples_params* params, int32_t* edge, double* error, double* distal, double* pendant,
                        int32_t* status) {
     if (!ctx) return -1;
+    const AltOut alt = take_alternatives(ctx);
     if (nq < 0 || (nq > 0 && (!packed_queries || !edge || !error || !distal || !pendant || !status)))
         return fail(ctx, "apples_place_batch: bad arguments");
     BatchIO io;
     io.h_queries = packed_queries;
     io.h_self = self_node;
     io.edge = edge; io.error = error; io.distal = distal; io.pendant = pendant; io.status = status;
+    io.alt = alt;
     return run_batch(ctx, nq, io, params);
 }
 
@@ -1356,6 +1424,7 @@ int apples_place_batch_bytes(apples_ctx* ctx, int64_t nq, const uint8_t* bytes, 
                              const int32_t* self_node, const apples_params* params, int32_t* edge, double* error,
                              double* distal, double* pendant, int32_t* status) {
     if (!ctx) return -1;
+    const AltOut alt = take_alternatives(ctx);
     if (ctx->kind < 0) return fail(ctx, "apples_set_reference has not been called");
     if (nq < 0 || (nq > 0 && (!bytes || row_stride < ctx->L || !edge || !error || !distal || !pendant || !status)))
         return fail(ctx, "apples_place_batch_bytes: bad arguments");
@@ -1364,6 +1433,7 @@ int apples_place_batch_bytes(apples_ctx* ctx, int64_t nq, const uint8_t* bytes, 
     io.byte_stride = row_stride;
     io.h_self = self_node;
     io.edge = edge; io.error = error; io.distal = distal; io.pendant = pendant; io.status = status;
+    io.alt = alt;
     return run_batch(ctx, nq, io, params);
 }
 
@@ -1414,12 +1484,14 @@ int apples_place_batch_matrix(apples_ctx* ctx, int64_t nq, const double* rows, c
                               const apples_params* params, int32_t* edge, double* error, double* distal,
                               double* pendant, int32_t* status) {
     if (!ctx) return -1;
+    const AltOut alt = take_alternatives(ctx);
     if (nq < 0 || (nq > 0 && (!rows || !edge || !error || !distal || !pendant || !status)))
         return fail(ctx, "apples_place_batch_matrix: bad arguments");
     BatchIO io;
     io.h_rows = rows;
     io.h_self = self_node;
     io.edge = edge; io.error = error; io.distal = distal; io.pendant = pendant; io.status = status;
+    io.alt = alt;
     return run_batch(ctx, nq, io, params);
 }
 

@@ -169,6 +169,15 @@ struct PlaceArgs {
     double* out_distal;
     double* out_pendant;
     int* out_status;
+    // ranked records (keep > 1, apples_set_alternatives): record j of query q at [q * keep + j], records 0 .. count[q] - 1
+    // in criterion order (record 0 = the placement above), unused slots edge -1 and zeros
+    int keep;
+    int* alt_count;
+    int* alt_edge;
+    double* alt_error;
+    double* alt_distal;
+    double* alt_pendant;
+    unsigned char* alt_int0;
     // optional per-edge export for one query (index inside the batch), arrays of M
     int dbg_query;
     double* dbg_x1;

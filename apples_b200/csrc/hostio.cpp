@@ -8,6 +8,7 @@
 //   apples_jplace_write   result arrays -> the jplace text `json.dumps(result, sort_keys=True, indent=4)` writes for the
 //                    joined per-query records (run_apples.py:106-118, jutil.py:1-19), byte for byte: Python float repr,
 //                    ensure_ascii string escapes, the "first record is kept even when unplaceable" quirk of join_jplace.
+//                    apples_jplace_write_k: the same with the ranked records of --keep-at-most K in each "p" list.
 //
 // Both are multi-threaded (std::thread): at config 5 the queries are 5 GB of text and a million records.  No CUDA kernel
 // is involved; cudaHostAlloc is used only to make the matrix directly DMA-able.
@@ -431,7 +432,21 @@ int apples_jplace_write(const char* path, const char* prefix, const char* suffix
                         const int64_t* name_off, const uint8_t* in_backbone, const int32_t* edge, const double* error,
                         const double* distal, const double* pendant, const int32_t* status, int exclude_intplace,
                         int n_threads, int64_t* n_written, char* err, int errlen) {
+    return apples_jplace_write_k(path, prefix, suffix, n, names, name_off, in_backbone, edge, error, distal, pendant, status,
+                                 exclude_intplace, 1, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n_threads,
+                                 n_written, err, errlen);
+}
+
+int apples_jplace_write_k(const char* path, const char* prefix, const char* suffix, int64_t n, const char* names,
+                          const int64_t* name_off, const uint8_t* in_backbone, const int32_t* edge, const double* error,
+                          const double* distal, const double* pendant, const int32_t* status, int exclude_intplace,
+                          int32_t keep, const int32_t* alt_count, const int32_t* alt_edge, const double* alt_error,
+                          const double* alt_distal, const double* alt_pendant, const uint8_t* alt_int0, int n_threads,
+                          int64_t* n_written, char* err, int errlen) {
     if (!path || !prefix || !suffix || n < 0 || (n > 0 && (!names || !name_off || !edge || !error || !distal || !pendant || !status)))
+        return -1;
+    if (keep < 1 || keep > APPLES_MAX_KEEP ||
+        (keep > 1 && n > 0 && (!alt_count || !alt_edge || !alt_error || !alt_distal || !alt_pendant || !alt_int0)))
         return -1;
     if (n_threads <= 0) n_threads = (int)std::max(1u, std::thread::hardware_concurrency());
     n_threads = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(n_threads, 64), (n + 4095) / 4096));
@@ -468,7 +483,22 @@ int apples_jplace_write(const char* path, const char* prefix, const char* suffix
             if (plain) out += '0'; else py_float_repr(distal[i], out);
             out += ",\n                    ";
             if (plain || (status[i] & APPLES_FLAG_PENDANT_INT0)) out += '0'; else py_float_repr(pendant[i], out);
-            out += "\n                ]\n            ]\n        }";
+            out += "\n                ]";
+            // records 1.. of a least-squares placement (keep > 1): like_weight_ratio 0
+            const int cnt = (keep > 1 && !plain && fe != -1) ? std::min<int32_t>(alt_count[i], keep) : 1;
+            for (int j = 1; j < cnt; ++j) {
+                const int64_t o = i * keep + j;
+                out += ",\n                [\n                    ";
+                out += std::to_string(alt_edge[o]);
+                out += ",\n                    ";
+                py_float_repr(alt_error[o], out);
+                out += ",\n                    0,\n                    ";
+                py_float_repr(alt_distal[o], out);
+                out += ",\n                    ";
+                if (alt_int0[o]) out += '0'; else py_float_repr(alt_pendant[o], out);
+                out += "\n                ]";
+            }
+            out += "\n            ]\n        }";
             counts[(size_t)t]++;
         }
     };

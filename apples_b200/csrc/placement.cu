@@ -252,6 +252,92 @@ __device__ __forceinline__ Work carve(unsigned char* base, int cap, int kcap) {
     return w;
 }
 
+// `cnt` ranked records of query q are written: the count, and edge -1 / zeros in the unused slots
+__device__ __forceinline__ void close_records(const PlaceArgs& a, int q, int cnt) {
+    a.alt_count[q] = cnt;
+    for (int j = cnt; j < a.keep; ++j) {
+        const size_t o = (size_t)q * a.keep + j;
+        a.alt_edge[o] = -1;
+        a.alt_error[o] = 0.0;
+        a.alt_distal[o] = 0.0;
+        a.alt_pendant[o] = 0.0;
+        a.alt_int0[o] = 0;
+    }
+}
+
+// The ranked records of one query (keep > 1), in the order of a stable sort by the criterion's key:
+//   MLSE / ME  the valid edges by (key, post-order index); record 0 is the argmin `first` of place_query.  keep - 1
+//              rounds of "next smallest (key, p) after the last one", each a solve of every edge and one group argmin;
+//   HYBRID     the nc candidates of place_query (hist[0 .. nc), in (error, index) order) by (x_1, candidate rank); one
+//              candidate per member of the group, keep rounds of the group argmin.  Record 0 is the first minimum of x_1.
+// S / R / len / orig are the query's working set over `cap` node slots (see Work).  (An out-of-line version raised the
+// registers of every kernel: 76 instead of 68.)
+template <class Coop>
+__device__ __forceinline__ void rank_records(const PlaceArgs& a, const int q, const double* S, const double* R,
+                                             const double* len, const int* orig, const int cap, const int* hist,
+                                             const int V, const int nc, const int first) {
+    constexpr int G = Coop::G;
+    const int lane = Coop::lane();
+    auto solve_at = [&](int p) {
+        double s[6], r[6];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) {
+            s[k] = S[k * cap + p];
+            r[k] = R[k * cap + p];
+        }
+        return solve_edge(s, r, len[p], a.negative_branch);
+    };
+    auto put = [&](int j, int p) {   // record j = edge p
+        const EdgeSol e = solve_at(p);
+        const size_t o = (size_t)q * a.keep + j;
+        a.alt_edge[o] = orig[p];
+        a.alt_error[o] = e.err;
+        a.alt_distal[o] = len[p] - e.x2;
+        a.alt_pendant[o] = e.x1;
+        a.alt_int0[o] = e.int0 ? 1 : 0;
+    };
+    int cnt = 0;
+    if (a.criterion == APPLES_HYBRID) {
+        Coop::sync();   // hist was written by member 0
+        double cx = 0.0;
+        if (lane < nc) cx = solve_at(hist[lane]).x1;
+        double last_x = 0.0;
+        int last_r = -1;
+        for (; cnt < a.keep; ++cnt) {
+            double v = 0.0;
+            int ix = 0x7fffffff;
+            if (lane < nc && (last_r < 0 || cx > last_x || (cx == last_x && lane > last_r))) { v = cx; ix = lane; }
+            Coop::argmin(v, ix);
+            if (ix == 0x7fffffff) break;
+            if (lane == 0) put(cnt, hist[ix]);
+            last_x = v;
+            last_r = ix;
+        }
+    } else {
+        const bool me = a.criterion == APPLES_ME;
+        if (lane == 0) put(0, first);
+        const EdgeSol e0 = solve_at(first);
+        double last_k = me ? e0.x1 : e0.err;
+        int last_p = first;
+        for (cnt = 1; cnt < a.keep; ++cnt) {
+            double v = 0.0;
+            int ix = 0x7fffffff;
+            for (int p = lane; p < V; p += G) {
+                const EdgeSol e = solve_at(p);
+                const double key = me ? e.x1 : e.err;
+                const bool after = key > last_k || (key == last_k && p > last_p);
+                if (after && (ix == 0x7fffffff || key < v)) { v = key; ix = p; }
+            }
+            Coop::argmin(v, ix);
+            if (ix == 0x7fffffff) break;
+            if (lane == 0) put(cnt, ix);
+            last_k = v;
+            last_p = ix;
+        }
+    }
+    if (lane == 0) close_records(a, q, cnt);
+}
+
 template <int METHOD, class Coop>
 __device__ __forceinline__ void place_query(const PlaceArgs& a, const int q, const int slot, const Work w, int* hist) {
     constexpr bool BME = METHOD == APPLES_BME;
@@ -469,6 +555,7 @@ __device__ __forceinline__ void place_query(const PlaceArgs& a, const int q, con
     Coop::argmin(bval, bidx);
     degenerate = Coop::any(degenerate);
     int best = bidx;
+    int nc = 0;   // HYBRID: candidates found
     if (a.criterion == APPLES_HYBRID) {
         // heapq.nsmallest(floor(log2 V), key=error) in (error, order) order, then the first minimum of x_1 among
         // them (Algorithm.py:77-82): floor(log2 V) rounds of "next smallest (error, index)"
@@ -486,12 +573,16 @@ __device__ __forceinline__ void place_query(const PlaceArgs& a, const int q, con
             }
             Coop::argmin(v, ix);
             if (ix == 0x7fffffff) break;
+            // rank_records re-sorts the candidates by x_1; the bucket table is free once the moments are done
+            if (a.keep > 1 && lane == 0) hist[nc] = ix;
+            ++nc;
             const double x1 = solve_at(ix).x1;
             if (best < 0 || x1 < best_x1) { best = ix; best_x1 = x1; }
             last_e = v;
             last_p = ix;
         }
     }
+    if (a.keep > 1) rank_records<Coop>(a, q, w.S, w.R, w.len, w.orig, cap, hist, V, nc, bidx);
     if (lane == 0) {
         const EdgeSol bs = solve_at(best);
         const double blen = w.len[best];
@@ -529,9 +620,11 @@ __global__ void __launch_bounds__(SmemClass<VCAP>::WARPS * 32) place_smem_kernel
     place_query<METHOD, WarpCoop>(a, q, a.slot_list ? a.slot_list[t] : q, w, hist);
 }
 
-// one block per query, working set in a global scratch region (rec_off / stack_off in node / chain slots)
+// one block per query, working set in a global scratch region (rec_off / stack_off in node / chain slots).  Three blocks
+// per SM (80 registers): without the bound the code of the ranked records would raise the register count of some methods
+// past it, or their spills
 template <int METHOD>
-__global__ void __launch_bounds__(PL_BLOCK_THREADS) place_block_kernel(const PlaceArgs a) {
+__global__ void __launch_bounds__(PL_BLOCK_THREADS, 3) place_block_kernel(const PlaceArgs a) {
     __shared__ int hist[PL_HIST + 1];
     const int t = blockIdx.x;
     const int q = a.qlist[t];
@@ -560,6 +653,15 @@ __global__ void finalize_kernel(const PlaceArgs a) {
     a.out_distal[q] = 0.0;
     a.out_pendant[q] = 0.0;
     a.out_status[q] = (st == ST_ZERO) ? APPLES_ZERO_DIST_LEAF : APPLES_TOO_FEW_DISTANCES;
+    if (a.keep > 1) {   // one record, the one above
+        const size_t o = (size_t)q * a.keep;
+        a.alt_edge[o] = a.out_edge[q];
+        a.alt_error[o] = 0.0;
+        a.alt_distal[o] = 0.0;
+        a.alt_pendant[o] = 0.0;
+        a.alt_int0[o] = 0;
+        close_records(a, q, 1);
+    }
 }
 
 // Sorts the batch's placeable queries into the launch classes on the device (the host would need two passes over the

@@ -94,12 +94,13 @@ def dumps(result):
 
 
 def write_arrays(output_fp, names, in_backbone, out, extended_newick_string, exclude_intplace=False, argv=None, threads=0,
-                 name_blob=None, name_off=None):
+                 name_blob=None, name_off=None, alt=None):
     """The fast path of run_apples.py's tail (join_jplace + json.dumps + write, run_apples.py:106-118) straight from the
     device result arrays, without a million per-query dicts: the native writer (apples_jplace_write, hostio.cpp) renders
     the "placements" list, Python renders the few lines around it.  Output is byte-identical to
     `write(assemble(results_to_jplace(...)))`.  `names` is a list of str, or pass the reader's NUL-separated UTF-8 blob
-    and offsets (FastaMatrix) as name_blob / name_off.  Returns the number of records written."""
+    and offsets (FastaMatrix) as name_blob / name_off.  alt: the ranked records of place_*(keep > 1), written as
+    results_to_jplace(..., alt=alt) lists them (apples_jplace_write_k).  Returns the number of placements written."""
     import ctypes as C
     import numpy as np
     from . import _lib
@@ -123,10 +124,17 @@ def write_arrays(output_fp, names, in_backbone, out, extended_newick_string, exc
     err = C.create_string_buffer(512)
     nw = C.c_int64(0)
     blob = C.create_string_buffer(name_blob, len(name_blob)) if not isinstance(name_blob, C.Array) else name_blob
-    rc = lib.apples_jplace_write(str(output_fp).encode(), head.encode(), (tail + '\n').encode(), n,
-                                 C.cast(blob, C.c_void_p), _lib.ptr(name_off), _lib.ptr(inb), _lib.ptr(edge), _lib.ptr(error),
-                                 _lib.ptr(distal), _lib.ptr(pendant), _lib.ptr(status), 1 if exclude_intplace else 0,
-                                 int(threads), C.byref(nw), err, 512)
+    args = (str(output_fp).encode(), head.encode(), (tail + '\n').encode(), n, C.cast(blob, C.c_void_p), _lib.ptr(name_off),
+            _lib.ptr(inb), _lib.ptr(edge), _lib.ptr(error), _lib.ptr(distal), _lib.ptr(pendant), _lib.ptr(status),
+            1 if exclude_intplace else 0)
+    if alt is None:
+        rc = lib.apples_jplace_write(*args, int(threads), C.byref(nw), err, 512)
+    else:
+        alt = [np.ascontiguousarray(a) for a in alt]
+        keep = int(alt[1].shape[1])
+        if any(a.shape[:1] != (n,) for a in alt) or any(a.shape[1:] != (keep,) for a in alt[1:]):
+            raise ValueError('write_arrays: the ranked records do not match the %d placements' % n)
+        rc = lib.apples_jplace_write_k(*args, keep, *[_lib.ptr(a) for a in alt], int(threads), C.byref(nw), err, 512)
     if rc != 0:
         raise OSError('writing %s failed: %s' % (output_fp, err.value.decode(errors='replace')))
     return int(nw.value)

@@ -3,7 +3,8 @@ apples/OptionsRun.py:5-112 and apples/OptionsBuild.py:4-10, plus two additions t
   --clusters FILE   TreeCluster-format TSV to use instead of running a clustering (TreeCluster.py is an external
                     dependency of the reference, Reference.py:87-88)
   --device N        first CUDA device ordinal (default 0); -T/--threads is accepted and ignored (no CPU workers);
-  --gpus N          GPUs to shard the queries over (0 = all visible: the analogue of upstream's -T 0 = all cores).
+  --gpus N          GPUs to shard the queries over (0 = all visible: the analogue of upstream's -T 0 = all cores);
+  --keep-at-most K  report the best K placements of each query (pplacer's name; default 1), ranked by the criterion.
 Backbone re-estimation with FastTree (reestimateBackbone.py) is outside the hot path: it is never run here, as with
 the reference's -D flag; without -D a warning says that results can differ from upstream's default.
 """
@@ -78,7 +79,12 @@ def options_config_run(argv=None):
                  help='masks low confidence characters in the alignments indicated by lowercase characters')
     p.add_option('--exclude', dest='exclude_intplace', action='store_true', default=False,
                  help='exclude queries placed on the internal nodes in jplace file.')
+    p.add_option('--keep-at-most', dest='keep_at_most', type=int, default=1, metavar='NUMBER',
+                 help='report the best NUMBER (1 to 16) placements of each query in criterion order; the extra ones have '
+                      'like_weight_ratio 0')
     options, args = _parse(p, argv)
+    if not 1 <= options.keep_at_most <= 16:
+        raise ValueError('--keep-at-most must be from 1 to 16, got %d' % options.keep_at_most)
     # OptionsRun.py:88-110
     if options.dist_fp:
         if options.ref_fp:

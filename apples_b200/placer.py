@@ -147,36 +147,55 @@ class GpuPlacer:
         return (np.empty(nq, np.int32), np.empty(nq, np.float64), np.empty(nq, np.float64), np.empty(nq, np.float64),
                 np.empty(nq, np.int32))
 
-    def place_packed(self, packed, self_node, params, out=None):
-        """packed queries (host) -> (edge, error, distal, pendant, status) arrays."""
+    @staticmethod
+    def _alt_outputs(nq, keep):
+        """ranked-record arrays: (count [nq], edge, error, distal, pendant, pendant_int0 [nq, keep])"""
+        return (np.empty(nq, np.int32), np.empty((nq, keep), np.int32), np.empty((nq, keep), np.float64),
+                np.empty((nq, keep), np.float64), np.empty((nq, keep), np.float64), np.empty((nq, keep), np.uint8))
+
+    def _register_alternatives(self, nq, keep, alt):
+        """keep > 1: the ranked-record arrays the next place call fills (apples_set_alternatives); None for keep 1"""
+        keep = check_keep(keep)
+        if keep == 1:
+            return None
+        alt = alt if alt is not None else self._alt_outputs(nq, keep)
+        self._check(self.lib.apples_set_alternatives(self.h, keep, *[_lib.ptr(a) for a in alt]))
+        return alt
+
+    def place_packed(self, packed, self_node, params, out=None, keep=1, alt=None):
+        """packed queries (host) -> (edge, error, distal, pendant, status) arrays.  keep > 1: returns (those arrays,
+        ranked records) with the records as _alt_outputs lays them out (record 0 = the placement of the five arrays)."""
         nq = int(packed.shape[0])
         out = out if out is not None else self._outputs(nq)
         packed = np.ascontiguousarray(packed)
+        alt = self._register_alternatives(nq, keep, alt)
         self._check(self.lib.apples_place_batch(self.h, nq, _lib.ptr(packed), _lib.ptr(self_node), _lib.C.byref(params),
                                                 *[_lib.ptr(o) for o in out]))
-        return out
+        return out if alt is None else (out, alt)
 
-    def place_bytes(self, mat, self_node, params, out=None):
-        """alignment bytes uint8 [nq, L] (host) -> result arrays; packing happens on the device."""
+    def place_bytes(self, mat, self_node, params, out=None, keep=1, alt=None):
+        """alignment bytes uint8 [nq, L] (host) -> result arrays; packing happens on the device.  keep: as place_packed."""
         if mat.shape[1] != self.L:
             raise ValueError('query alignment has %d columns, reference has %d' % (mat.shape[1], self.L))
         if not (mat.dtype == np.uint8 and mat.ndim == 2 and mat.strides[1] == 1 and mat.strides[0] >= mat.shape[1]):
             mat = np.ascontiguousarray(mat, dtype=np.uint8)
         nq = int(mat.shape[0])
         out = out if out is not None else self._outputs(nq)
+        alt = self._register_alternatives(nq, keep, alt)
         # rows may be padded (the native reader's matrix: row stride = L rounded up to 16): the stride is passed on
         self._check(self.lib.apples_place_batch_bytes(self.h, nq, mat.ctypes.data, mat.strides[0] if nq else self.L,
                                                       _lib.ptr(self_node), _lib.C.byref(params), *[_lib.ptr(o) for o in out]))
-        return out
+        return out if alt is None else (out, alt)
 
-    def place_rows(self, rows, self_node, params, out=None):
-        """distance-matrix rows float64 [nq, n_cols] -> result arrays."""
+    def place_rows(self, rows, self_node, params, out=None, keep=1, alt=None):
+        """distance-matrix rows float64 [nq, n_cols] -> result arrays.  keep: as place_packed."""
         rows = np.ascontiguousarray(rows, dtype=np.float64)
         nq = int(rows.shape[0])
         out = out if out is not None else self._outputs(nq)
+        alt = self._register_alternatives(nq, keep, alt)
         self._check(self.lib.apples_place_batch_matrix(self.h, nq, _lib.ptr(rows), _lib.ptr(self_node),
                                                        _lib.C.byref(params), *[_lib.ptr(o) for o in out]))
-        return out
+        return out if alt is None else (out, alt)
 
     def upload_queries(self, packed, self_node=None):
         packed = np.ascontiguousarray(packed) if isinstance(packed, np.ndarray) else packed
@@ -258,8 +277,11 @@ class GpuPlacer:
         return x1, x2, err, valid
 
 
-def results_to_jplace(names, in_backbone, out, exclude_intplace=False, log=True, degenerate='raise'):
+def results_to_jplace(names, in_backbone, out, exclude_intplace=False, log=True, degenerate='raise', alt=None):
     """Device result arrays -> the per-query dicts PoolQueryWorker.runquery returns, with its messages.
+
+    alt: the ranked records of place_*(keep > 1).  A query placed by least squares (PLACED, or PLACED_MISPLACEMENT_FLAG
+    without exclude_intplace) then carries its count records in 'p', records 1.. with like_weight_ratio 0.
 
     degenerate='raise' (default): a query whose status carries APPLES_FLAG_DEGENERATE raises ZeroDivisionError, as the
     reference does in util.solve2_2 (util.py:26-27: `1 / (a_11 * a_22 - a_12 * a_21)`, `assert det != 0`), where the
@@ -311,7 +333,23 @@ def results_to_jplace(names, in_backbone, out, exclude_intplace=False, log=True,
                                     'an internal node with a non-zero least squares error. This is a potential '
                                     'misplacement.%s' % (name, ignored))
         results[i] = {'placements': [{'p': [p], 'n': [name]}]}
+    if alt is not None:
+        cnt, a_edge, a_err, a_distal, a_pend, a_int0 = alt
+        code = st_arr & _lib.STATUS_CODE_MASK
+        ls = (code == _lib.PLACED) | ((code == _lib.PLACED_MISPLACEMENT_FLAG) & (not exclude_intplace))
+        for i in np.flatnonzero(ls & (np.asarray(cnt) > 1)).tolist():
+            p = results[i]['placements'][0]['p']
+            for j in range(1, int(cnt[i])):
+                p.append([int(a_edge[i, j]), float(a_err[i, j]), 0, float(a_distal[i, j]),
+                          0 if a_int0[i, j] else float(a_pend[i, j])])
     return results
+
+
+def check_keep(keep):
+    """--keep-at-most K: 1 <= K <= 16 (APPLES_MAX_KEEP)"""
+    if isinstance(keep, bool) or int(keep) != keep or not 1 <= keep <= _lib.MAX_KEEP:
+        raise ValueError('--keep-at-most must be an integer from 1 to %d, got %r' % (_lib.MAX_KEEP, keep))
+    return int(keep)
 
 
 class MultiGpuPlacer:
@@ -352,29 +390,31 @@ class MultiGpuPlacer:
             p.set_matrix_tags(tags)
         self.matrix_tags = self.placers[0].matrix_tags
 
-    def _sharded(self, method, mat, self_node, params):
+    def _sharded(self, method, mat, self_node, params, keep):
         from .parallel import shard_bounds
         nq = int(mat.shape[0])
         out = self.placers[0]._outputs(nq)
+        alt = self.placers[0]._alt_outputs(nq, check_keep(keep)) if keep > 1 else None
         bounds = shard_bounds(nq, len(self.placers))
 
         def run(i):
             b, e = bounds[i]
             if e > b:
                 part = getattr(self.placers[i], method)(mat[b:e], None if self_node is None else self_node[b:e], params,
-                                                        out=tuple(o[b:e] for o in out))
-                assert part[0].ctypes.data == out[0][b:e].ctypes.data
+                                                        out=tuple(o[b:e] for o in out), keep=keep,
+                                                        alt=None if alt is None else tuple(a[b:e] for a in alt))
+                assert (part if alt is None else part[0])[0].ctypes.data == out[0][b:e].ctypes.data
         list(self.pool.map(run, range(len(self.placers))))
-        return out
+        return out if alt is None else (out, alt)
 
-    def place_bytes(self, mat, self_node, params):
+    def place_bytes(self, mat, self_node, params, keep=1):
         if not (mat.dtype == np.uint8 and mat.ndim == 2 and mat.strides[1] == 1):
             mat = np.ascontiguousarray(mat, dtype=np.uint8)
-        return self._sharded('place_bytes', mat, self_node, params)
+        return self._sharded('place_bytes', mat, self_node, params, keep)
 
-    def place_rows(self, rows, self_node, params):
+    def place_rows(self, rows, self_node, params, keep=1):
         rows = np.ascontiguousarray(rows, dtype=np.float64)
-        return self._sharded('place_rows', rows, self_node, params)
+        return self._sharded('place_rows', rows, self_node, params, keep)
 
     def timings(self, reset=False):
         """Stage timers of the contexts: times are the maximum over the GPUs (they run side by side), counters the sum."""
@@ -405,11 +445,12 @@ def _distributed_world():
     return 0, 1
 
 
-def place_arrays(reference, options, name_to_node_map, queries, tree=None, placer=None, device=0, devices=None):
+def place_arrays(reference, options, name_to_node_map, queries, tree=None, placer=None, device=0, devices=None, keep=1):
     """The device part of place_batch: returns (names, in_backbone, (edge, error, distal, pendant, status)) for ALL
-    queries in input order.  Inside an initialised torch.distributed job every rank places its contiguous block of
+    queries in input order, and the ranked records as a fourth item when keep > 1 (GpuPlacer.place_packed).  Inside an initialised torch.distributed job every rank places its contiguous block of
     ceil(Q / world) queries on its own GPU and the blocks are exchanged with one all-gather of 32-byte records
     (apples_b200.parallel); otherwise the queries are sharded over `devices` inside this process."""
+    keep = check_keep(keep)
     names = [q[0] for q in queries]
     rank, world = _distributed_world()
     lo, hi = 0, len(queries)
@@ -456,16 +497,16 @@ def place_arrays(reference, options, name_to_node_map, queries, tree=None, place
                 else:
                     for t, v in q[2].items():
                         rows[i, col[t]] = v
-            out = placer.place_rows(rows, self_node, params) if mine else placer._outputs(0)
+            res = placer.place_rows(rows, self_node, params, keep=keep) if mine else _empty_outputs(placer, keep)
         else:
             params = placer.params_from_options(options, reference)
             mat = _fasta.as_byte_matrix([q[1] for q in mine], placer.L)
-            out = placer.place_bytes(mat, self_node, params) if mine else placer._outputs(0)
+            res = placer.place_bytes(mat, self_node, params, keep=keep) if mine else _empty_outputs(placer, keep)
         log_stage_times(placer, len(mine), t_before)
         if world > 1:
             from .parallel import gather_placements
-            out = gather_placements(out, len(queries))
-        return names, in_backbone, out
+            res = gather_placements(res, len(queries)) if keep == 1 else gather_placements(res[0], len(queries), alt=res[1])
+        return (names, in_backbone, res) if keep == 1 else (names, in_backbone) + tuple(res)
     finally:
         if own:
             placer.close()
@@ -512,11 +553,14 @@ def log_messages(names, in_backbone, out, exclude_intplace=False):
                             'misplacement.%s' % (name, ignored))
 
 
-def place_alignment(reference, options, name_to_node_map, names, mat, tree=None, placer=None, device=0, devices=None):
+def place_alignment(reference, options, name_to_node_map, names, mat, tree=None, placer=None, device=0, devices=None,
+                    keep=1):
     """Array-level twin of place_batch for alignment input: `names` (list of str) and `mat` (uint8 [n, L] alignment bytes
     as fasta2dic / the native reader leave them, e.g. FastaMatrix.matrix).  Returns (in_backbone, (edge, error, distal,
     pendant, status)) for all queries in input order -- no per-query Python objects, so a million queries cost
-    milliseconds of host time.  Sharding over `devices` / torch.distributed ranks as in place_arrays."""
+    milliseconds of host time -- and the ranked records as a third item when keep > 1 (GpuPlacer.place_packed).
+    Sharding over `devices` / torch.distributed ranks as in place_arrays."""
+    keep = check_keep(keep)
     rank, world = _distributed_world()
     n = len(names)
     lo, hi = 0, n
@@ -543,18 +587,23 @@ def place_alignment(reference, options, name_to_node_map, names, mat, tree=None,
         params = placer.params_from_options(options, reference)
         if mat.shape[1] != placer.L:
             raise ValueError('query alignment has %d columns, reference has %d' % (mat.shape[1], placer.L))
-        out = placer.place_bytes(mat[lo:hi], self_node, params) if hi > lo else placer._outputs(0)
+        res = placer.place_bytes(mat[lo:hi], self_node, params, keep=keep) if hi > lo else _empty_outputs(placer, keep)
         log_stage_times(placer, hi - lo, t_before)
         if world > 1:
             from .parallel import gather_placements
-            out = gather_placements(out, n)
-        return in_backbone, out
+            res = gather_placements(res, n) if keep == 1 else gather_placements(res[0], n, alt=res[1])
+        return (in_backbone, res) if keep == 1 else (in_backbone,) + tuple(res)
     finally:
         if own:
             placer.close()
 
 
-def place_batch(reference, options, name_to_node_map, queries, tree=None, placer=None, device=0, devices=None):
+def _empty_outputs(placer, keep):
+    out = placer._outputs(0)
+    return out if keep == 1 else (out, GpuPlacer._alt_outputs(0, keep))
+
+
+def place_batch(reference, options, name_to_node_map, queries, tree=None, placer=None, device=0, devices=None, keep=1):
     """Drop-in for `pool.starmap(queryworker.runquery, queries)` (run_apples.py:94-102).
 
     queries yields (query_name, query_seq 'S1' row or None, obs_dist dict or None) exactly as run_apples.py builds
@@ -562,11 +611,15 @@ def place_batch(reference, options, name_to_node_map, queries, tree=None, placer
     `tree` is the BackboneTree the name_to_node_map belongs to (or pass an existing GpuPlacer / MultiGpuPlacer).
     `devices` = list of CUDA ordinals to shard the queries over (default: the single `device`); the result does not
     depend on it.  Under torchrun (torch.distributed initialised) every rank returns the full list.
+    keep > 1 (--keep-at-most): the 'p' list of a query placed by least squares holds its best `keep` placements in
+    criterion order (results_to_jplace).
     """
     queries = list(queries)
     if not queries:
         return []
-    names, in_backbone, out = place_arrays(reference, options, name_to_node_map, queries, tree=tree, placer=placer,
-                                           device=device, devices=devices)
+    keep = check_keep(keep)
+    names, in_backbone, out, *alt = place_arrays(reference, options, name_to_node_map, queries, tree=tree, placer=placer,
+                                                 device=device, devices=devices, keep=keep)
     log = _distributed_world()[0] == 0   # messages once per job
-    return results_to_jplace(names, in_backbone, out, getattr(options, 'exclude_intplace', False), log=log)
+    return results_to_jplace(names, in_backbone, out, getattr(options, 'exclude_intplace', False), log=log,
+                             alt=alt[0] if alt else None)

@@ -124,6 +124,20 @@ int apples_place_batch_bytes(apples_ctx* ctx, int64_t nq, const uint8_t* bytes, 
                              const int32_t* self_node, const apples_params* params, int32_t* edge, double* error,
                              double* distal, double* pendant, int32_t* status);
 
+/* Ranked records (pplacer's --keep-at-most): the best `keep` placements of every query, ranked on the device by the
+ * criterion -- a stable sort of the valid edges by the criterion's key in edge_index order, truncated to keep (MLSE: error,
+ * ME: x_1; HYBRID: the floor(log2 V) candidates of the smallest error sorted by x_1, so at most that many records).
+ * Registers caller-owned host buffers that the NEXT apples_place_batch / _bytes / _matrix call fills, beside its usual
+ * outputs; that call takes the registration (also when it fails), so it serves one call.  count[nq]; edge, error,
+ * distal, pendant and pendant_int0 (1 where the pendant is the Python int 0, as APPLES_FLAG_PENDANT_INT0) are
+ * [nq][keep]: record j of query q at q * keep + j for j < count[q].  Record 0 is the placement the call returns in its
+ * own outputs.  Queries that are not placed by least squares (APPLES_ZERO_DIST_LEAF, APPLES_TOO_FEW_DISTANCES) have
+ * count 1.  Unused slots hold edge -1 and zeros.  1 <= keep <= APPLES_MAX_KEEP; keep = 1 or six NULL buffers clear the
+ * registration.  One call beside the three place calls instead of three twins of them: their signatures stay. */
+#define APPLES_MAX_KEEP 16
+int apples_set_alternatives(apples_ctx* ctx, int32_t keep, int32_t* count, int32_t* edge, double* error, double* distal,
+                            double* pendant, uint8_t* pendant_int0);
+
 /* The hot path, distance-matrix input: rows is double[nq][n_cols] (run_apples.py:43-54). */
 int apples_place_batch_matrix(apples_ctx* ctx, int64_t nq, const double* rows, const int32_t* self_node,
                               const apples_params* params, int32_t* edge, double* error, double* distal,
@@ -213,6 +227,16 @@ int apples_jplace_write(const char* path, const char* prefix, const char* suffix
                         const int64_t* name_off, const uint8_t* in_backbone, const int32_t* edge, const double* error,
                         const double* distal, const double* pendant, const int32_t* status, int exclude_intplace,
                         int n_threads, int64_t* n_written, char* err, int errlen);
+/* The same with the ranked records of apples_set_alternatives: a query placed by least squares (status APPLES_PLACED, or
+ * APPLES_PLACED_MISPLACEMENT_FLAG without exclude_intplace) gets alt_count[i] records in "p", record 0 from the five
+ * arrays as above, records 1.. from alt_*[i * keep + j] with like_weight_ratio 0.  Every other query keeps its single
+ * record.  keep = 1 (alt_* may be NULL) writes exactly what apples_jplace_write writes. */
+int apples_jplace_write_k(const char* path, const char* prefix, const char* suffix, int64_t n, const char* names,
+                          const int64_t* name_off, const uint8_t* in_backbone, const int32_t* edge, const double* error,
+                          const double* distal, const double* pendant, const int32_t* status, int exclude_intplace,
+                          int32_t keep, const int32_t* alt_count, const int32_t* alt_edge, const double* alt_error,
+                          const double* alt_distal, const double* alt_pendant, const uint8_t* alt_int0, int n_threads,
+                          int64_t* n_written, char* err, int errlen);
 
 /* Newick text -> flat post-order arrays, replacing treeswift.read_tree_newick + index_edges + set_levels
  * (apples/prepareTree.py:24, apples/util.py:57-88): node id = edge_index = post-order rank (children left to right, root

@@ -124,12 +124,15 @@ def main(argv=None):
     startq = time.time()
     if queries is not None:
         # distance-matrix input: the per-query dict interface of the reference (pool.starmap(runquery) drop-in)
-        results = place_batch(reference, options, name_to_node_map, queries, tree=tree, devices=devices)
+        results = place_batch(reference, options, name_to_node_map, queries, tree=tree, devices=devices,
+                              keep=options.keep_at_most)
         n_q = len(queries)
     else:
         # alignment input: byte matrix -> result arrays -> jplace text, all native
-        in_backbone, out = place_alignment(reference, options, name_to_node_map, q_names, q_mat, tree=tree, devices=devices) \
+        in_backbone, out, *alt = place_alignment(reference, options, name_to_node_map, q_names, q_mat, tree=tree,
+                                                 devices=devices, keep=options.keep_at_most) \
             if len(q_names) else (np.zeros(0, bool), None)
+        alt = alt[0] if alt else None   # ranked records (--keep-at-most > 1)
         n_q = len(q_names)
     logging.info('[%s] Processed all queries in %.3f seconds on %d GPU(s).' % (time.strftime('%H:%M:%S'),
                                                                                time.time() - startq, max(world, len(devices))))
@@ -144,10 +147,11 @@ def main(argv=None):
         else:
             log_messages(q_names, in_backbone, out, options.exclude_intplace)
             if options.output_fp:
-                jplace.write_arrays(options.output_fp, q_names, in_backbone, out, extended_newick_string, options.exclude_intplace)
+                jplace.write_arrays(options.output_fp, q_names, in_backbone, out, extended_newick_string, options.exclude_intplace,
+                                    alt=alt)
             else:
                 from apples_b200.placer import results_to_jplace
-                res = results_to_jplace(q_names, in_backbone.tolist(), out, options.exclude_intplace, log=False)
+                res = results_to_jplace(q_names, in_backbone.tolist(), out, options.exclude_intplace, log=False, alt=alt)
                 jplace.write(jplace.assemble(res, extended_newick_string), None)
         LAST_TIMINGS['write_s'] = time.time() - startw
         LAST_TIMINGS['total_s'] = time.time() - startb
