@@ -83,7 +83,7 @@ def load():
     lib.apples_results_download.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_results_to_device.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.apples_distance_counts.argtypes = [vp, i64, vp, dbl, vp, vp, vp]
-    lib.apples_count_keys.argtypes = [vp, i64, vp, C.POINTER(Params), C.POINTER(i32), vp]
+    lib.apples_count_keys.argtypes = [vp, i64, vp, C.POINTER(Params), C.POINTER(i32), vp, vp]
     lib.apples_observed_sets.argtypes = [vp, i64, vp, vp, vp, C.POINTER(Params), i32, vp, vp, vp]
     lib.apples_edge_solutions.argtypes = [vp, vp, vp, i32, C.POINTER(Params), vp, vp, vp, vp]
     lib.apples_get_timings.argtypes = [vp, vp, C.c_int, C.c_int]

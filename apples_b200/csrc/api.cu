@@ -83,6 +83,7 @@ struct apples_ctx {
     // per-batch work buffers
     DevBuf q_rm, q_wm, keys, self_node, obs_node, obs_dist, obs_len, obs_len2, Kd, Vd, statusd, zero_edge, pair_counter;
     DevBuf q_bytes, q_bytes2, q_rm2, bad_flag, clk_probe, stash_keys, stash_ids, stash_count;
+    DevBuf kmin, stash_kmin;   // line minima of keys / stash_keys (nucleotide count keys)
     double dense_mhz = 0.0;  // effective SM clock of the last dense launch (clock64 / globaltimer of CTA 0)
     DevBuf obs_node2, obs_dist2, qlist, pl_lists, bin_counts, bin_lists, rec_off, stack_off, recs, stacks;
     DevBuf o_edge, o_err, o_distal, o_pendant, o_status;
@@ -98,7 +99,7 @@ struct apples_ctx {
     std::vector<TimedSpan> spans;
     std::vector<cudaEvent_t> ev_pool;
     double t_ms[T_NSTAGE] = {0, 0, 0, 0, 0, 0};
-    double n_launch = 0, n_dense_launch = 0, n_pairs = 0, n_obs = 0, n_valid = 0, n_over = 0, max_K = 0, max_V = 0;
+    double n_launch = 0, n_dense_launch = 0, n_pairs = 0, n_lines = 0, n_obs = 0, n_valid = 0, n_over = 0, max_K = 0, max_V = 0;
     size_t scratch_limit = (size_t)6 << 30;  // placement scratch pool upper bound (bytes)
     int64_t max_subbatch = 65536;
     int64_t max_batch = 1 << 20;  // queries per macro-batch (batch-wide observed-list buffers)
@@ -373,6 +374,7 @@ struct BatchIO {
     // count-keys export: every sub-batch's [nb][n_rep] block of the key matrix is copied to h_keys and the batch stops
     // after the count stage (no selection, no placement)
     void* h_keys = nullptr;
+    uint32_t* h_kmin = nullptr;   // optional: their line minima [nq][ceil(n_rep / 32)] (nucleotide count keys only)
     bool stop_after_count = false;
     double* dbg_x1 = nullptr; double* dbg_x2 = nullptr; double* dbg_err = nullptr; uint8_t* dbg_valid = nullptr;
     AltOut alt;   // ranked records [nq][alt.keep] when alt.keep > 1 (host output only)
@@ -509,6 +511,7 @@ struct MacroBatch {
     // work buffers of the batch (grown, never shrunk), the zeroing of its counters and flags, and the self-node upload
     int allocate() {
         if (ensure(ctx, ctx->keys, (size_t)(use_tc ? round_up(QB, 256) : QB) * ldk * key_bytes)) return -1;
+        if (sel_kind == SEL_NUC && ensure(ctx, ctx->kmin, (size_t)(use_tc ? round_up(QB, 256) : QB) * (ldk / 32) * 4)) return -1;
         if (use_tc && ensure(ctx, ctx->q_img, dense_tc_image_bytes(round_up(QB, 256), ctx->tc_nw))) return -1;
         if (io.h_bytes) {
             if (ensure(ctx, ctx->q_bytes, (size_t)QB * io.byte_stride) || ensure(ctx, ctx->bad_flag, 4)) return -1;
@@ -541,7 +544,7 @@ struct MacroBatch {
         if (ensure(ctx, ctx->Kd, (size_t)n * 4) || ensure(ctx, ctx->Vd, (size_t)n * 4) ||
             ensure(ctx, ctx->statusd, (size_t)n * 4) || ensure(ctx, ctx->zero_edge, (size_t)n * 4))
             return -1;
-        if (ensure(ctx, ctx->pair_counter, 8)) return -1;
+        if (ensure(ctx, ctx->pair_counter, 16)) return -1;   // member distances, key lines read
         if (ensure(ctx, ctx->o_edge, (size_t)n * 4) || ensure(ctx, ctx->o_err, (size_t)n * 8) ||
             ensure(ctx, ctx->o_distal, (size_t)n * 8) || ensure(ctx, ctx->o_pendant, (size_t)n * 8) ||
             ensure(ctx, ctx->o_status, (size_t)n * 4))
@@ -556,7 +559,7 @@ struct MacroBatch {
         if (ensure(ctx, ctx->rec_off, (size_t)(n + 1) * 8) || ensure(ctx, ctx->stack_off, (size_t)(n + 1) * 8) ||
             ensure(ctx, ctx->qlist, (size_t)std::max(n, 1) * 4) || ensure(ctx, ctx->pl_lists, (size_t)std::max(n, 1) * 8))
             return -1;
-        CK(cudaMemsetAsync(ctx->pair_counter.p, 0, 8, s));
+        CK(cudaMemsetAsync(ctx->pair_counter.p, 0, 16, s));
         if (ensure(ctx, ctx->bin_counts, 64) || ensure(ctx, ctx->bin_lists, (size_t)PLACE_NCLASS * std::max(n, 1) * 4)) return -1;
         CK(cudaMemsetAsync(ctx->bin_counts.p, 0, 64, s));
         if (io.dbg_x1) {
@@ -583,8 +586,8 @@ struct MacroBatch {
         // key-row stash for the overflow reruns (alignment-mode nucleotides): up to 256 MiB of key rows
         if (sel_kind == SEL_NUC && !matrix) {
             stash_cap = (int)std::min<int64_t>(n, std::max<int64_t>(1, ((int64_t)256 << 20) / (ldk * 4)));
-            if (ensure(ctx, ctx->stash_keys, (size_t)stash_cap * ldk * 4) || ensure(ctx, ctx->stash_ids, (size_t)stash_cap * 4) ||
-                ensure(ctx, ctx->stash_count, 4))
+            if (ensure(ctx, ctx->stash_keys, (size_t)stash_cap * ldk * 4) || ensure(ctx, ctx->stash_kmin, (size_t)stash_cap * (ldk / 32) * 4) ||
+                ensure(ctx, ctx->stash_ids, (size_t)stash_cap * 4) || ensure(ctx, ctx->stash_count, 4))
                 return -1;
             CK(cudaMemsetAsync(ctx->stash_count.p, 0, 4, s));
         }
@@ -596,6 +599,7 @@ struct MacroBatch {
         sa.ldk = ldk;
         sa.keys_nuc = (const uint32_t*)ctx->keys.p;
         sa.keys_f64 = (const double*)ctx->keys.p;
+        sa.kmin = (const uint32_t*)ctx->kmin.p;
         sa.goff = (const int*)ctx->goff.p;
         sa.gmem = (const int*)ctx->gmem.p;
         sa.ref_node = (const int*)ctx->ref_node.p;
@@ -620,6 +624,7 @@ struct MacroBatch {
         sa.tree = tree_dev(ctx);
         if (stash_cap > 0) {
             sa.stash_keys = (uint32_t*)ctx->stash_keys.p;
+            sa.stash_kmin = (uint32_t*)ctx->stash_kmin.p;
             sa.stash_ids = (int*)ctx->stash_ids.p;
             sa.stash_count = (int*)ctx->stash_count.p;
             sa.stash_cap = stash_cap;
@@ -630,6 +635,7 @@ struct MacroBatch {
         sa.obs_dist = r.dist;
         sa.obs_len = r.len;
         sa.pair_counter = (unsigned long long*)ctx->pair_counter.p;
+        sa.line_counter = (unsigned long long*)ctx->pair_counter.p + 1;
 
         const bool dbg = io.dbg_x1 != nullptr;
         pa.K = (const int*)ctx->Kd.p;
@@ -684,6 +690,11 @@ struct MacroBatch {
                 const size_t row = (size_t)n_units * key_bytes;
                 CK(cudaMemcpy2DAsync((char*)io.h_keys + (size_t)(base0 + sb0) * row, row, ctx->keys.p, (size_t)ldk * key_bytes,
                                      row, nb, cudaMemcpyDeviceToHost, s));
+                if (io.h_kmin && sel_kind == SEL_NUC && !slow_ctx) {
+                    const size_t mrow = (size_t)((n_units + 31) / 32) * 4;
+                    CK(cudaMemcpy2DAsync((char*)io.h_kmin + (size_t)(base0 + sb0) * mrow, mrow, ctx->kmin.p, (size_t)(ldk / 32) * 4,
+                                         mrow, nb, cudaMemcpyDeviceToHost, s));
+                }
             } else {
                 SelectArgs a = sa;
                 a.q_begin = sb0;
@@ -750,8 +761,8 @@ struct MacroBatch {
         return 0;
     }
 
-    // count stage of `nb` queries on stream st: their key rows (row stride ldk) into ctx->keys.  d_q = their packed rows;
-    // matrix rows are their own keys.  slow: byte-compare fallback, d_qb = the queries' padded byte rows [nb][Lp], 64-bit keys
+    // count stage of `nb` queries on stream st: their key rows (row stride ldk) into ctx->keys, and for packed nucleotide
+    // keys their line minima into ctx->kmin.  d_q = their packed rows; matrix rows are their own keys.  slow: byte-compare fallback, d_qb = the queries' padded byte rows [nb][Lp], 64-bit keys
     // into kw
     int count(cudaStream_t st, const void* d_q, int nb, bool slow, const uint8_t* d_qb, void* kw) {
         if (slow) {
@@ -772,7 +783,7 @@ struct MacroBatch {
             {
                 Span sp(ctx, T_DENSE, st);
                 launch_dense_tc(ctx->q_img.p, q_pad, ctx->reps_img.p, ctx->tc_rep_pad, ctx->tc_nw, (uint32_t*)ctx->keys.p, ldk,
-                                ctx->num_sms, st);
+                                (uint32_t*)ctx->kmin.p, sa.gate.vmin, ctx->num_sms, st);
                 ctx->n_launch += 1;
                 ctx->n_dense_launch += 1;
                 ctx->n_tc_launch += 1;
@@ -792,7 +803,8 @@ struct MacroBatch {
                                       (const uint32_t*)ctx->reps_wm.p, (const uint32_t*)ctx->reps_nv.p, ctx->rep_pad,
                                       ctx->W, ctx->Wp, (uint32_t*)ctx->keys.p, ldk, (unsigned long long*)ctx->clk_probe.p,
                                       ctx->num_sms, st);
-                ctx->n_launch += 1;
+                launch_line_minima((const uint32_t*)ctx->keys.p, nb, ldk, sa.gate.vmin, (uint32_t*)ctx->kmin.p, st);
+                ctx->n_launch += 2;
                 ctx->n_dense_launch += 1;
             }
             ctx->n_pairs += (double)nb * ctx->n_rep;
@@ -1013,11 +1025,15 @@ struct MacroBatch {
                 a.obs_dist = r.dist;
                 a.obs_len = r.len;
                 a.pair_counter = nullptr;
+                a.line_counter = nullptr;
                 a.stash_keys = nullptr;
                 const void* d_q = matrix ? nullptr : ctx->q_rm.p;
                 const uint8_t* d_qb = (const uint8_t*)ctx->q_bytes_p.p;
                 void* kw = slow_ctx ? ctx->keys.p : ctx->keys_w.p;
-                if (use_st) a.keys_nuc = (const uint32_t*)ctx->stash_keys.p + (size_t)o0 * ldk;
+                if (use_st) {
+                    a.keys_nuc = (const uint32_t*)ctx->stash_keys.p + (size_t)o0 * ldk;
+                    a.kmin = (const uint32_t*)ctx->stash_kmin.p + (size_t)o0 * (ldk / 32);
+                }
                 else if (count(ss, d_q, ng, slow, d_qb, kw)) return -1;
                 if (select(ss, a, d_q, ng, slow, d_qb, kw)) return -1;
                 mark("  rerun select launched");
@@ -1190,9 +1206,10 @@ struct MacroBatch {
             CK(cudaMemcpy(io.dbg_err, ctx->dbg_err.p, (size_t)ctx->M * 8, cudaMemcpyDeviceToHost));
             CK(cudaMemcpy(io.dbg_valid, ctx->dbg_valid.p, (size_t)ctx->M, cudaMemcpyDeviceToHost));
         }
-        unsigned long long pc = 0;
-        CK(cudaMemcpy(&pc, ctx->pair_counter.p, 8, cudaMemcpyDeviceToHost));
-        ctx->n_pairs += (double)pc;
+        unsigned long long pc[2] = {0, 0};
+        CK(cudaMemcpy(pc, ctx->pair_counter.p, 16, cudaMemcpyDeviceToHost));
+        ctx->n_pairs += (double)pc[0];
+        ctx->n_lines += (double)pc[1];
         if (sel_kind == SEL_NUC && !matrix && ctx->clk_probe.p) {
             unsigned long long c[4] = {0, 0, 0, 0};
             CK(cudaMemcpy(c, ctx->clk_probe.p, 32, cudaMemcpyDeviceToHost));
@@ -1634,7 +1651,7 @@ int apples_distance_counts(apples_ctx* ctx, int64_t nq, const void* packed_queri
 }
 
 int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, const apples_params* params,
-                      int32_t* key_kind, void* keys) {
+                      int32_t* key_kind, void* keys, uint32_t* line_minima) {
     if (!ctx) return -1;
     if (ctx->kind < 0) return fail(ctx, "apples_set_reference has not been called");
     if (nq <= 0 || !packed_queries || !key_kind || !keys) return fail(ctx, "apples_count_keys: bad arguments");
@@ -1642,6 +1659,7 @@ int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, c
     BatchIO io;
     io.h_queries = packed_queries;
     io.h_keys = keys;
+    io.h_kmin = *key_kind == 0 ? line_minima : nullptr;
     io.stop_after_count = true;
     return run_batch(ctx, nq, io, params);
 }
@@ -1693,14 +1711,14 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
 
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset) {
     if (!ctx || !out) return -1;
-    double v[22] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
+    double v[23] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
                     ctx->t_ms[T_D2H], ctx->n_launch, ctx->n_dense_launch, ctx->n_pairs, ctx->n_obs, ctx->n_valid,
                     ctx->n_over, ctx->max_K, ctx->max_V, ctx->dense_mhz, ctx->n_place_class[0], ctx->n_place_class[1],
-                    ctx->n_place_class[2], ctx->n_place_class[3], ctx->n_place_class[4], ctx->n_slow, ctx->n_tc_launch};
-    for (int i = 0; i < n && i < 22; ++i) out[i] = v[i];
+                    ctx->n_place_class[2], ctx->n_place_class[3], ctx->n_place_class[4], ctx->n_slow, ctx->n_tc_launch, ctx->n_lines};
+    for (int i = 0; i < n && i < 23; ++i) out[i] = v[i];
     if (reset) {
         for (int i = 0; i < T_NSTAGE; ++i) ctx->t_ms[i] = 0;
-        ctx->n_launch = ctx->n_dense_launch = ctx->n_pairs = ctx->n_obs = ctx->n_valid = ctx->n_over = ctx->max_K = ctx->max_V = 0;
+        ctx->n_launch = ctx->n_dense_launch = ctx->n_pairs = ctx->n_lines = ctx->n_obs = ctx->n_valid = ctx->n_over = ctx->max_K = ctx->max_V = 0;
         for (int c = 0; c < PLACE_NCLASS; ++c) ctx->n_place_class[c] = 0;
         ctx->n_slow = 0;
         ctx->n_tc_launch = 0;

@@ -78,6 +78,30 @@ __device__ __forceinline__ double jc69_from_counts(uint32_t m, uint32_t v, int v
     return -0.75 * log(loc);
 }
 
+// ---- per-line key minima (count stage -> selection).  A line is the 32 keys [32 l, 32 l + 32) of a key row; its minimum
+// is the key of smallest ratio m / v among the keys the selection can use (v >= max(vmin, 1) and 4 m < 3 v, the gate of
+// classify() in select.cu), the smallest column on equal ratios, or LINE_NONE when no key of the line is usable.  A pure
+// function of the keys: both count kernels fold it with these two helpers.
+constexpr uint32_t LINE_NONE = 1u;   // m = 1, v = 0: compares greater than every usable key
+
+// the key itself when the selection can use it, LINE_NONE otherwise (vmin1 = max(vmin, 1))
+__device__ __forceinline__ uint32_t line_usable(uint32_t k, uint32_t vmin1) {
+    const uint32_t m = k & 0xffffu, v = k >> 16;
+    return (v >= vmin1 && 4u * m < 3u * v) ? k : LINE_NONE;
+}
+// the smaller ratio of two usable-or-LINE_NONE keys, exactly (counts <= 65535: products fit 32 bits); a = the smaller column
+__device__ __forceinline__ uint32_t line_min2(uint32_t a, uint32_t b) {
+    return (b & 0xffffu) * (a >> 16) < (a & 0xffffu) * (b >> 16) ? b : a;
+}
+// minimum of 32 consecutive keys (k[j] = column 32 l + j, already passed through line_usable): a pairwise tree, left wins ties
+__device__ __forceinline__ uint32_t line_min32(uint32_t* k) {
+#pragma unroll
+    for (int s = 1; s < 32; s <<= 1)
+#pragma unroll
+        for (int j = 0; j < 32; j += 2 * s) k[j] = line_min2(k[j], k[j + s]);
+    return k[0];
+}
+
 // scoredist from the BLOSUM45 sum and the valid count (distance.py:699-712)
 __device__ __forceinline__ double scoredist_from_sum(double tot, uint32_t v, int L, double overlap) {
     if (v == 0u || (double)v / (double)L < overlap) return -1.0;
@@ -100,6 +124,7 @@ struct SelectArgs {
     int n_units;           // representatives (alignment) or matrix columns
     int64_t ldk;           // row stride of the key matrix
     const uint32_t* keys_nuc;  // [nq][ldk] packed (mismatch | valid << 16)
+    const uint32_t* kmin;      // SEL_NUC: [nq][ldk / 32] line minima of keys_nuc (LINE_NONE etc., see above)
     const double* keys_f64;    // [nq][ldk] distances (protein representatives / matrix rows); SEL_NUCW: 64-bit count keys
     const int* goff;       // cluster CSR
     const int* gmem;
@@ -130,10 +155,12 @@ struct SelectArgs {
     int* status;           // [nq] ST_*
     int* zero_edge;        // [nq]
     unsigned long long* pair_counter;  // number of member distances evaluated (statistics)
+    unsigned long long* line_counter;  // SEL_NUC: number of key lines loaded (statistics)
     // key-row stash (nucleotide alignment mode, first pass only): a query that overflows its slot copies its key row
     // aside so that its rerun needs no second distance pass.  stash_count is bumped for every overflowing query; only
     // the first stash_cap of them are stored (the host falls back to recomputing when there are more)
     uint32_t* stash_keys;  // [stash_cap][ldk] or NULL
+    uint32_t* stash_kmin;  // [stash_cap][ldk / 32] their line minima
     int* stash_ids;        // [stash_cap] query index inside the batch
     int* stash_count;
     int stash_cap;
@@ -193,6 +220,7 @@ void launch_row_valid(const uint32_t* rm, int rows, int W, uint32_t* nv, int row
 void launch_dense_nuc_keys(const uint32_t* q_wm, const uint32_t* q_nv, int q_pad, const uint32_t* r_wm,
                            const uint32_t* r_nv, int r_pad, int W, int Wp, uint32_t* keys, int64_t ldk,
                            unsigned long long* clk, int num_sms, cudaStream_t s);
+void launch_line_minima(const uint32_t* keys, int rows, int64_t ldk, int vmin, uint32_t* kmin, cudaStream_t s);
 void launch_dense_nuc_full(const uint32_t* q_wm, const uint32_t* q_nv, int q_pad, int nq, const uint32_t* r_wm,
                            const uint32_t* r_nv, int r_pad, int n_ref, int W, int Wp, int vmin, uint32_t* mism, uint32_t* valid,
                            double* dist, int num_sms, cudaStream_t s);
@@ -213,8 +241,8 @@ int dense_tc_max_sites();
 int dense_tc_tile_rows();
 size_t dense_tc_image_bytes(int rows_pad, int n_w);
 void launch_tc_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int vw, void* out, cudaStream_t s);
-void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk, int num_sms,
-                     cudaStream_t s);
+void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
+                     uint32_t* kmin, int vmin, int num_sms, cudaStream_t s);
 cudaError_t launch_pack(int kind, const uint8_t* bytes, int64_t row_stride, int n, int L, void* out, int* bad, cudaStream_t s,
                         int* row_flag = nullptr);
 cudaError_t launch_repitch_bytes(const uint8_t* src, int64_t src_stride, int n, int L, int Lp, uint8_t* dst, cudaStream_t s);

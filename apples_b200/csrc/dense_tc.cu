@@ -15,7 +15,8 @@
 // 0.78 of its pipe roofline (DESIGN.md section 3a): the stage is compute-bound, so it belongs on the tensor cores.
 //
 // Kernel: persistent, one CTA per SM: warp 0 = TMA producer (1-D bulk copies of pre-arranged operand images), warp 1 = MMA
-// issuer (one thread), warps 2-9 = epilogue (tcgen05.ld, decode, 32-bit keys identical to distance.cu's).
+// issuer (one thread), warps 2-9 = epilogue (tcgen05.ld, decode, 32-bit keys identical to distance.cu's, and the line
+// minima of those keys, common.cuh).
 // CTA tile 256 queries x 256 representatives = two M=128, N=256 accumulators (all 512 TMEM columns) sharing the B operand in
 // shared memory, 3 stages of 32 sites (128 bytes of K per row: A 32 KB + B 32 KB).  Operands are K-major, no swizzle: an
 // operand image is [k16 = 8][row block = 32][8 rows][16 bytes], i.e. 128-byte core matrices with SBO = 128 B between row
@@ -141,6 +142,8 @@ struct TcArgs {
     int q_pad, r_pad, n_w;
     uint32_t* keys;         // [q_pad][ldk] (mismatch | valid << 16)
     int64_t ldk;
+    uint32_t* kmin;         // [q_pad][ldk / 32] line minima of the keys (common.cuh)
+    uint32_t vmin1;         // max(vmin, 1): the overlap gate of the line minima
     int sq, sr;             // super-tile shape (query tiles x representative tiles) of the L2-friendly tile order
 };
 
@@ -249,6 +252,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a)
 #pragma unroll 1
             for (int h = 0; h < 2; ++h) {
                 const int row0 = qt * TC_TM + h * 128 + quarter * 32;   // first of the warp's 32 rows
+                // the minima of the lane's row in the warp's 4 lines, shifted in one line per 32 columns
+                uint32_t lm0 = LINE_NONE, lm1 = LINE_NONE, lm2 = LINE_NONE, lm3 = LINE_NONE;
 #pragma unroll 1
                 for (int c = c0; c < c0 + TC_TN / 2; c += 32) {
                     uint32_t v[32];
@@ -266,14 +271,26 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a)
                     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
                     // decode, then transpose the warp's 32 rows x 32 columns through shared memory: a lane holds one ROW of
                     // the block, but a store instruction should write whole 128-byte row segments (4 rows x 128 B per
-                    // instruction instead of 32 rows x 16 B: 8x fewer lines per store)
+                    // instruction instead of 32 rows x 16 B: 8x fewer lines per store).
+                    // The line minimum in registers: the lane holds the whole line of its row (no shuffles).  Folded on
+                    // (mismatch, match) in column order: m / v orders as m / match, and a key under the overlap gate never
+                    // replaces the running minimum (which starts at "none", 1 / 0); whether the winner passes 4 m < 3 v is
+                    // decided once per line below.  Same result as line_usable / line_min32 (common.cuh)
+                    uint32_t bmi = 1u, bma = 0u;
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
                         const int S = (int)v[j];
                         const uint32_t match = (uint32_t)(S + (TC_W - 1)) / (uint32_t)TC_W;
                         const uint32_t mism = (uint32_t)((int)((TC_W - 1) * match) - S);
                         xp[lane * 33 + j] = mism | ((match + mism) << 16);
+                        const bool lower = match + mism >= a.vmin1 && mism * bma < bmi * match;
+                        bmi = lower ? mism : bmi;
+                        bma = lower ? match : bma;
                     }
+                    lm0 = lm1;
+                    lm1 = lm2;
+                    lm2 = lm3;
+                    lm3 = (bmi < 3u * bma) ? (bmi | ((bmi + bma) << 16)) : LINE_NONE;
                     __syncwarp();
 #pragma unroll
                     for (int r0 = 0; r0 < 32; r0 += 4) {
@@ -284,6 +301,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a)
                     }
                     __syncwarp();
                 }
+                // one 16-byte store per row: lines (rt * 256 + c0) / 32 .. + 3 (ldk is a multiple of 256)
+                __stcs(reinterpret_cast<uint4*>(a.kmin + (size_t)(row0 + lane) * (a.ldk / 32) + ((size_t)rt * TC_TN + c0) / 32),
+                       make_uint4(lm0, lm1, lm2, lm3));
             }
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
@@ -305,8 +325,8 @@ int dense_tc_max_sites() { return TC_MAX_L; }
 int dense_tc_tile_rows() { return TC_TM; }
 size_t dense_tc_image_bytes(int rows_pad, int n_w) { return (size_t)(rows_pad / TC_TM) * n_w * TC_IMG; }
 
-void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk, int num_sms,
-                     cudaStream_t s) {
+void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
+                     uint32_t* kmin, int vmin, int num_sms, cudaStream_t s) {
     TcArgs a;
     a.a_img = (const uint8_t*)a_img;
     a.b_img = (const uint8_t*)b_img;
@@ -315,6 +335,8 @@ void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad,
     a.n_w = n_w;
     a.keys = keys;
     a.ldk = ldk;
+    a.kmin = kmin;
+    a.vmin1 = (uint32_t)(vmin > 1 ? vmin : 1);
     // super-tiles of about one wave: 12 x 12 tiles = 144 CTAs share 12 + 12 operand images per K step (shapes from 7 x 7 to
     // 37 x 4 measure within 2% of each other, profiles/tc_tile_sweep_r02.txt; only 1-wide strips lose, 11%)
     a.sq = 12;

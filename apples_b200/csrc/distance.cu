@@ -393,6 +393,32 @@ void launch_dense_nuc_keys(const uint32_t* q_wm, const uint32_t* q_nv, int q_pad
     dense_nuc_kernel<false><<<dense_grid(q_pad, r_pad, num_sms), DT_THREADS, DT_SMEM_BYTES, s>>>(a);
 }
 
+// line minima of a key block written by dense_nuc_kernel<false> (the tensor-core kernel folds them in its epilogue): one
+// thread per line, the same helpers, so the two count paths agree bit for bit
+__global__ void __launch_bounds__(256) line_minima_kernel(const uint32_t* __restrict__ keys, int rows, int64_t ldk, uint32_t vmin1,
+                                                          uint32_t* __restrict__ kmin) {
+    const int64_t nl = ldk / 32;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)rows * nl) return;
+    const uint4* src = reinterpret_cast<const uint4*>(keys + i * 32);   // row r, line l starts at r * ldk + 32 l = 32 i
+    uint32_t k[32];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const uint4 x = src[j];
+        k[4 * j] = line_usable(x.x, vmin1);
+        k[4 * j + 1] = line_usable(x.y, vmin1);
+        k[4 * j + 2] = line_usable(x.z, vmin1);
+        k[4 * j + 3] = line_usable(x.w, vmin1);
+    }
+    kmin[i] = line_min32(k);
+}
+
+void launch_line_minima(const uint32_t* keys, int rows, int64_t ldk, int vmin, uint32_t* kmin, cudaStream_t s) {
+    const int64_t n = (int64_t)rows * (ldk / 32);
+    if (n <= 0) return;
+    line_minima_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(keys, rows, ldk, (uint32_t)(vmin > 1 ? vmin : 1), kmin);
+}
+
 void launch_dense_nuc_full(const uint32_t* q_wm, const uint32_t* q_nv, int q_pad, int nq, const uint32_t* r_wm,
                            const uint32_t* r_nv, int r_pad, int n_ref, int W, int Wp,
                            int vmin, uint32_t* mism, uint32_t* valid, double* dist, int num_sms,

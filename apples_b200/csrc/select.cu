@@ -10,6 +10,8 @@
 // used both keys re-scans its residue class for the next two) until obs_num reaches baseobs.  The scan is branch-free
 // per key (two multiplies, one compare); the exact classification runs only for the few keys that can matter.  A query
 // whose observed set outgrows its slot stashes its key row and is rerun with a larger slot (HEAVY instantiation).
+// select_nuc_kernel reaches the same set without the full scan: it reads only the key lines that the count stage's
+// line minima call for (see the kernel).
 // Two kernels: select_nuc_kernel for the packed nucleotide counts of the dense kernels (the hot path), select_kernel for
 // the byte-compare fallback (SEL_NUCW), protein (SEL_AA) and distance-matrix (SEL_MATRIX) inputs.
 // Nucleotide keys are the exact integer pairs (mismatch, valid) from the dense kernel: ordering by the rational
@@ -758,6 +760,9 @@ __global__ void __launch_bounds__(32 * SEL_GEN_WARPS, 16 / SEL_GEN_WARPS) select
 #ifndef SEL_HEAVY_WARPS
 #define SEL_HEAVY_WARPS 1
 #endif
+// shared 32-bit words per warp: `words` for the queue, the member list and the sort, then one byte per key line
+__host__ __device__ inline int sel_nuc_warp_words(int words, int n_units) { return words + (n_units + 127) / 128; }
+
 template <bool HEAVY>
 __global__ void __launch_bounds__(32 * (HEAVY ? SEL_HEAVY_WARPS : SEL_NUC_WARPS), (HEAVY ? 16 : 32) / (HEAVY ? SEL_HEAVY_WARPS : SEL_NUC_WARPS))
 select_nuc_kernel(const SelectArgs a) {
@@ -772,7 +777,7 @@ select_nuc_kernel(const SelectArgs a) {
     constexpr int PF = HEAVY ? 16 : SEL_PF;     // rows prefetched ahead of the one being counted
     constexpr int POS_BITS = 27;
     extern __shared__ uint32_t s_sortbuf[];
-    uint32_t* wbuf = s_sortbuf + (threadIdx.x >> 5) * WORDS;
+    uint32_t* wbuf = s_sortbuf + (threadIdx.x >> 5) * sel_nuc_warp_words(WORDS, a.n_units);
     int* queue = reinterpret_cast<int*>(wbuf);
     int* lrow = reinterpret_cast<int*>(wbuf + QCAP);
     uint32_t* lmeta = wbuf + QCAP + LCAP;
@@ -794,15 +799,66 @@ select_nuc_kernel(const SelectArgs a) {
     st.znode = -1;
     st.zkey.idx = 0;
 
-#ifndef SEL_U
-#define SEL_U 8
-#endif
-    constexpr int U = SEL_U;   // keys per lane and chunk (independent loads in flight)
-    Key<KIND> l1 = key_none<KIND>(), l2 = key_none<KIND>();
-    uint32_t bm = 1u, bv = 0u;
-    int u0 = 0, np = 0, qhead = 0;
-    bool scan_done = a.n_units <= 0, far_init = false, more = false;
-    unsigned long long pairs = 0ull;
+    // ---- the key row is read line by line (32 keys, one 128-byte load), driven by the line minima of the count stage
+    // (common.cuh).  Near phase: the minima row is read 32 lines at a time and only the lines whose minimum could be near
+    // (ratio below the guard band's upper edge P_hi / 65536; the LINE_NONE minimum never is, and nothing is when P_hi =
+    // 0) are opened: their near keys go to the queue, their smallest far key becomes the line's entry.  A line that is
+    // not opened holds no near key (its usable keys all have a ratio >= its minimum's).  Far phase: an exact lazy merge
+    // over the lines, in (ratio, index) order.  The entry of a line not opened is its minimum with index 32 l, a lower
+    // bound of every key of the line under key_less; the entry of an opened line is its smallest far key after the last
+    // one taken.  The warp-wide smallest entry is either a bound (the line is opened, its entry replaced) or the next far
+    // unit (queued and expanded as before; its line's entry becomes the line's next far key).  Lane o keeps the smallest
+    // entry of the lines l with l % 32 == o; after a line of lane o changes, the warp recomputes that minimum (one
+    // entry per lane).  The per-line state lives in shared memory, one byte per line after the WORDS of the queue:
+    // LS_UNOPENED, the position (0..31) of the line's current far key, or LS_DONE. ----
+    constexpr uint8_t LS_UNOPENED = 0xff, LS_DONE = 32;
+    uint8_t* lst = reinterpret_cast<uint8_t*>(wbuf + WORDS);
+    const int n_kl = (a.n_units + 31) >> 5;
+    const uint32_t* __restrict__ mrow = a.kmin + (size_t)slot * (size_t)(a.ldk >> 5);
+    // entry of line l (every lane may ask for a different line)
+    auto line_entry = [&](int l) -> Key<KIND> {
+        const uint32_t ls = lst[l];
+        if (ls == LS_UNOPENED) {
+            const uint32_t mk = mrow[l];
+            return mk == LINE_NONE ? key_none<KIND>() : make_key<KIND>(mk, 32 * l);
+        }
+        return ls < 32u ? make_key<KIND>(krow[32 * l + ls], 32 * l + (int)ls) : key_none<KIND>();
+    };
+    // the smallest far key of line l after g (after nothing: all = true), the same on every lane; lane 0 records its position
+    auto load_line = [&](int l, const Key<KIND>& g, bool all, int& cls) -> Key<KIND> {
+        const int u = 32 * l + lane;
+        const Key<KIND> k = make_key<KIND>(u < a.n_units ? krow[u] : 0u, u);
+        cls = classify(a, k);
+        Key<KIND> f = (cls == 2 && (all || key_less(g, k))) ? k : key_none<KIND>();
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const Key<KIND> of = key_shfl_xor(f, o);
+            if (key_less(of, f)) f = of;
+        }
+        if (lane == 0) lst[l] = key_is_none(f) ? LS_DONE : (uint8_t)(f.idx & 31);
+        __syncwarp();
+        return f;
+    };
+    // the smallest entry of the lines of lane `owner`, computed by the warp
+    auto class_min = [&](int owner) -> Key<KIND> {
+        Key<KIND> b = key_none<KIND>();
+        for (int l = owner + 32 * lane; l < n_kl; l += 32 * 32) {
+            const Key<KIND> e = line_entry(l);
+            if (key_less(e, b)) b = e;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const Key<KIND> ob = key_shfl_xor(b, o);
+            if (key_less(ob, b)) b = ob;
+        }
+        return b;
+    };
+
+    Key<KIND> best = key_none<KIND>();   // far phase: the smallest entry of this lane's lines
+    int l0 = 0, cl0 = 0, np = 0, qhead = 0;
+    unsigned cand = 0u;                   // lines cl0 + t of the current chunk of minima still to be opened
+    bool scan_done = n_kl <= 0, far_init = false;
+    unsigned long long pairs = 0ull, lines_read = 0ull;
 
     for (;;) {
         if (np < 32 && !scan_done) {
@@ -813,64 +869,28 @@ select_nuc_kernel(const SelectArgs a) {
             if (lane < np) queue[lane] = keep;
             qhead = 0;
             do {
-                // ---- one chunk of the scan.  Event test per key, branch-free: ratio m / v below the lane's bound, the
-                // larger of the band's upper edge P_hi / 65536 and the ratio of l2 (l2.m << 16 and P_hi * v fit 32 bits:
-                // counts <= 65535, P_hi < 49154) ----
-                {
-#ifndef SEL_KPF
-#define SEL_KPF 2   // key chunks prefetched ahead of the one being scanned
-#endif
-                    const int u = u0 + SEL_KPF * 32 * U + lane * 32;
-                    if (lane < U && u < a.n_units) prefetch_l2(krow + u);
+                if (cand == 0u) {
+                    // ---- the next 32 line minima ----
+                    const int l = l0 + lane;
+                    if (lane == 0 && l0 + 64 < n_kl) prefetch_l2(mrow + l0 + 64);
+                    const uint32_t mk = l < n_kl ? mrow[l] : LINE_NONE;
+                    if (l < n_kl) lst[l] = LS_UNOPENED;
+                    cand = __ballot_sync(FULLMASK, ((mk & 0xffffu) << 16) < a.gate.P_hi * (mk >> 16));
+                    cl0 = l0;
+                    l0 += 32;
+                    __syncwarp();
+                } else {
+                    // ---- open one line: near keys to the queue (at most 32 on top of fewer than 32 left over) ----
+                    const int l = cl0 + __ffs(cand) - 1;
+                    cand &= cand - 1;
+                    int cls;
+                    load_line(l, key_none<KIND>(), true, cls);
+                    const unsigned bal = __ballot_sync(FULLMASK, cls == 1);
+                    if (cls == 1) queue[np + __popc(bal & ((1u << lane) - 1u))] = 32 * l + lane;
+                    np += __popc(bal);
+                    ++lines_read;
                 }
-                uint32_t raw[U];
-#pragma unroll
-                for (int j = 0; j < U; ++j) {
-                    const int u = u0 + j * 32 + lane;
-                    raw[j] = 0;
-                    if (u < a.n_units) raw[j] = krow[u];
-                }
-                unsigned ev = 0u;
-#pragma unroll
-                for (int j = 0; j < U; ++j) {
-                    const uint32_t r = raw[j], m = r & 0xffffu, v = r >> 16;
-                    if (m * bv < bm * v) ev |= 1u << j;
-                }
-                unsigned nearb = 0u;
-                if (__any_sync(FULLMASK, ev != 0u)) {
-                    while (ev) {
-                        const int j = __ffs(ev) - 1;
-                        ev &= ev - 1;
-                        uint32_t rj = raw[0];
-#pragma unroll
-                        for (int t = 1; t < U; ++t)
-                            if (j == t) rj = raw[t];
-                        const Key<KIND> kj = make_key<KIND>(rj, u0 + j * 32 + lane);
-                        const int c = classify(a, kj);
-                        if (c == 1) nearb |= 1u << j;
-                        if (c == 2 && key_less(kj, l2)) {
-                            if (key_less(kj, l1)) {
-                                l2 = l1;
-                                l1 = kj;
-                            } else {
-                                l2 = kj;
-                            }
-                        }
-                    }
-                    const bool far_rules = (l2.m << 16) > a.gate.P_hi * l2.v;
-                    bm = far_rules ? l2.m : a.gate.P_hi;
-                    bv = far_rules ? l2.v : 65536u;
-                }
-                if (__any_sync(FULLMASK, nearb != 0u)) {
-#pragma unroll
-                    for (int j = 0; j < U; ++j) {
-                        const unsigned bal = __ballot_sync(FULLMASK, (nearb >> j) & 1u);
-                        if ((nearb >> j) & 1u) queue[np + __popc(bal & ((1u << lane) - 1u))] = u0 + j * 32 + lane;
-                        np += __popc(bal);
-                    }
-                }
-                u0 += 32 * U;
-                scan_done = u0 >= a.n_units;
+                scan_done = l0 >= n_kl && cand == 0u;
             } while (np < 32 && !scan_done);
             __syncwarp();
         }
@@ -878,67 +898,35 @@ select_nuc_kernel(const SelectArgs a) {
             // ---- the scan is over and every near unit is expanded: far units, ascending, while obs_num < baseobs ----
             if (!(st.obs_num < a.baseobs && st.kcount <= a.cap)) break;
             if (!far_init) {
-                more = !key_is_none(l2);  // the class may hold far keys beyond the two kept
+                for (int l = lane; l < n_kl; l += 32) {
+                    const Key<KIND> e = line_entry(l);
+                    if (key_less(e, best)) best = e;
+                }
                 far_init = true;
             }
-            Key<KIND> g = l1;
+            for (;;) {
+                Key<KIND> g = best;
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const Key<KIND> og = key_shfl_xor(g, o);
-                if (key_less(og, g)) g = og;
-            }
-            if (key_is_none(g)) break;  // no far unit left
-            const bool mine = l1.idx == g.idx;
-            if (mine) {
-                l1 = l2;
-                l2 = key_none<KIND>();
-            }
-            const unsigned refill = __ballot_sync(FULLMASK, mine && more && key_is_none(l1));
-            if (refill) {
-                const int owner = __ffs(refill) - 1;
-                Key<KIND> n1 = key_none<KIND>(), n2 = key_none<KIND>();
-                constexpr int RU = 4;
-                for (int k0 = lane; k0 * 32 < a.n_units; k0 += 32 * RU) {
-                    uint32_t rr[RU];
-#pragma unroll
-                    for (int j = 0; j < RU; ++j) {
-                        const int u = (k0 + 32 * j) * 32 + owner;
-                        rr[j] = 0;
-                        if (u < a.n_units) rr[j] = krow[u];
-                    }
-#pragma unroll
-                    for (int j = 0; j < RU; ++j) {
-                        const int u = (k0 + 32 * j) * 32 + owner;
-                        const Key<KIND> kj = make_key<KIND>(rr[j], u);
-                        if (u < a.n_units && classify(a, kj) == 2 && key_less(g, kj) && key_less(kj, n2)) {
-                            if (key_less(kj, n1)) {
-                                n2 = n1;
-                                n1 = kj;
-                            } else {
-                                n2 = kj;
-                            }
-                        }
-                    }
+                for (int o = 16; o > 0; o >>= 1) {
+                    const Key<KIND> og = key_shfl_xor(g, o);
+                    if (key_less(og, g)) g = og;
                 }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {  // merge the sorted pairs
-                    const Key<KIND> b1 = key_shfl_xor(n1, o), b2 = key_shfl_xor(n2, o);
-                    if (key_less(b1, n1)) {
-                        n2 = key_less(n1, b2) ? n1 : b2;
-                        n1 = b1;
-                    } else if (key_less(b1, n2)) {
-                        n2 = b1;
-                    }
-                }
-                if (lane == owner) {
-                    l1 = n1;
-                    l2 = n2;
-                    more = !key_is_none(n2);
+                if (key_is_none(g)) break;  // no far unit left
+                const int l = g.idx >> 5;
+                const bool bound = lst[l] == LS_UNOPENED;
+                int cls;
+                load_line(l, g, bound, cls);   // opens the line, or moves its entry past g
+                lines_read += bound ? 1ull : 0ull;
+                const Key<KIND> nb = class_min(l & 31);
+                if (lane == (l & 31)) best = nb;
+                if (!bound) {
+                    if (lane == 0) queue[0] = g.idx;
+                    qhead = 0;
+                    np = 1;
+                    break;
                 }
             }
-            if (lane == 0) queue[0] = g.idx;
-            qhead = 0;
-            np = 1;
+            if (np == 0) break;
             __syncwarp();
         }
         // ---- expand up to 32 pending units: lane t owns unit t ----
@@ -1005,6 +993,7 @@ select_nuc_kernel(const SelectArgs a) {
         if (st.kcount > a.cap) break;
     }
     if (lane == 0 && a.pair_counter && pairs) atomicAdd(a.pair_counter, pairs);
+    if (lane == 0 && a.line_counter && lines_read) atomicAdd(a.line_counter, lines_read);
 
     // ---- PoolQueryWorker.runquery:72-98 (as in select_kernel) ----
     int status = ST_PLACE;
@@ -1019,6 +1008,8 @@ select_nuc_kernel(const SelectArgs a) {
                 const uint4* src = reinterpret_cast<const uint4*>(krow);
                 uint4* dst = reinterpret_cast<uint4*>(a.stash_keys + (size_t)pos * a.ldk);
                 for (int64_t x = lane; x < a.ldk / 4; x += 32) dst[x] = src[x];
+                uint32_t* mdst = a.stash_kmin + (size_t)pos * (size_t)(a.ldk >> 5);
+                for (int64_t x = lane; x < (a.ldk >> 5); x += 32) mdst[x] = mrow[x];
                 if (lane == 0) a.stash_ids[pos] = gid;
             }
         }
@@ -1075,12 +1066,14 @@ void launch_select(int kind, const SelectArgs& a, cudaStream_t s) {
     if (a.n <= 0) return;
     if (kind == SEL_NUC && a.out_map) {  // overflow rerun
         const int w = SEL_HEAVY_WARPS;
-        const size_t sm = (size_t)w * 4096 * 4;   // select_nuc_kernel<true>: WORDS per warp
+        const size_t sm = (size_t)w * sel_nuc_warp_words(4096, a.n_units) * 4;   // select_nuc_kernel<true>: WORDS = 4096
         cudaFuncSetAttribute(select_nuc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         select_nuc_kernel<true><<<(a.n + w - 1) / w, w * 32, sm, s>>>(a);
     } else if (kind == SEL_NUC) {
         const int w = SEL_NUC_WARPS;
-        select_nuc_kernel<false><<<(a.n + w - 1) / w, w * 32, (size_t)w * 1024 * 4, s>>>(a);
+        const size_t sm = (size_t)w * sel_nuc_warp_words(1024, a.n_units) * 4;
+        cudaFuncSetAttribute(select_nuc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        select_nuc_kernel<false><<<(a.n + w - 1) / w, w * 32, sm, s>>>(a);
     } else {
         const int w = SEL_GEN_WARPS;
         const dim3 g((a.n + w - 1) / w), b(w * 32);

@@ -221,12 +221,12 @@ class GpuPlacer:
         return K, V, ov
 
     def timings(self, reset=False):
-        v = np.zeros(22, np.float64)
-        self.lib.apples_get_timings(self.h, _lib.ptr(v), 22, 1 if reset else 0)
+        v = np.zeros(23, np.float64)
+        self.lib.apples_get_timings(self.h, _lib.ptr(v), 23, 1 if reset else 0)
         keys = ['h2d_ms', 'transpose_ms', 'rep_distance_ms', 'selection_ms', 'placement_ms', 'd2h_ms', 'launches',
                 'rep_distance_launches', 'pairs', 'observed', 'valid_nodes', 'overflow_queries', 'max_observed',
                 'max_valid_nodes', 'rep_distance_sm_mhz', 'placed_smem64', 'placed_smem128', 'placed_smem256',
-                'placed_smem512', 'placed_block', 'fallback_queries', 'tensor_core_launches']
+                'placed_smem512', 'placed_block', 'fallback_queries', 'tensor_core_launches', 'key_lines_read']
         return dict(zip(keys, v.tolist()))
 
     # ------------------------------------------------------------------------------------------------ parity exports
@@ -240,17 +240,22 @@ class GpuPlacer:
                                                     _lib.ptr(valid), _lib.ptr(dist)))
         return mism, valid, dist
 
-    def count_keys(self, packed, params):
+    def count_keys(self, packed, params, line_minima=False):
         """Query x representative keys of the hot path's count stage (apples_count_keys): ([nq, n_rep] array, kind) with
-        kind 0 = uint32 mismatch | valid << 16, 1 = uint64 mismatch | valid << 32 (byte mode), 2 = float64 scoredist."""
+        kind 0 = uint32 mismatch | valid << 16, 1 = uint64 mismatch | valid << 32 (byte mode), 2 = float64 scoredist.
+        line_minima=True appends the [nq, ceil(n_rep / 32)] uint32 line minima (None unless kind is 0)."""
         packed = np.ascontiguousarray(packed)
         nq = int(packed.shape[0])
         raw = np.zeros(nq * self.n_rep, np.uint64)
+        mins = np.zeros((nq, (self.n_rep + 31) // 32), np.uint32) if line_minima else None
         kind = _lib.C.c_int32(-1)
         self._check(self.lib.apples_count_keys(self.h, nq, _lib.ptr(packed), _lib.C.byref(params), _lib.C.byref(kind),
-                                               _lib.ptr(raw)))
+                                               _lib.ptr(raw), _lib.ptr(mins) if line_minima else None))
         dtype = {0: np.uint32, 1: np.uint64, 2: np.float64}[kind.value]
-        return raw.view(dtype)[:nq * self.n_rep].reshape(nq, self.n_rep), kind.value
+        keys = raw.view(dtype)[:nq * self.n_rep].reshape(nq, self.n_rep)
+        if line_minima:
+            return keys, kind.value, (mins if kind.value == 0 else None)
+        return keys, kind.value
 
     def observed_sets(self, params, packed=None, rows=None, self_node=None, cap=4096):
         src = packed if packed is not None else rows

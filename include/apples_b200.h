@@ -165,9 +165,13 @@ int apples_distance_counts(apples_ctx* ctx, int64_t nq, const void* packed_queri
  *   0  uint32  mismatch | valid << 16   (tensor-core or integer-pipe kernel)
  *   1  uint64  mismatch | valid << 32   (byte-compare fallback: L > 65 535 or bytes other than A,C,G,T,- in the reference)
  *   2  double  scoredist with params->overlap_frac (APPLES_AA)
- * The caller sizes keys for 8 bytes per entry unless it knows the context's kind. */
+ * The caller sizes keys for 8 bytes per entry unless it knows the context's kind.
+ * line_minima (optional, NULL = not wanted; written for kind 0 only) is [nq][ceil(n_rep / 32)]: per line of 32 keys
+ * [32 l, 32 l + 32), the key of smallest ratio mismatch / valid among the keys with valid >= max(vmin, 1) and
+ * 4 mismatch < 3 valid (vmin: the smallest valid count that passes params->overlap_frac), the smallest column on equal
+ * ratios, or 0x00000001 when no key of the line qualifies.  The selection reads only the lines these minima call for. */
 int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, const apples_params* params,
-                      int32_t* key_kind, void* keys);
+                      int32_t* key_kind, void* keys, uint32_t* line_minima);
 
 /* kernel (c): the observed set of each query as the reference would hold it after PoolQueryWorker.py:40-70 (self
  * entry removed), sorted by node id; count[q] may exceed cap (then only cap entries are written).
@@ -193,7 +197,8 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
  * [14] effective SM clock in MHz during the last representative-distance launch (clock64 / globaltimer, in-kernel)
  * [15..19] queries placed by the shared-memory placement launches of 64 / 128 / 256 / 512 node slots and by the
  * block-per-query launch (global scratch)  [20] queries that went through the byte-compare fallback
- * [21] representative-distance launches that ran on the tensor cores */
+ * [21] representative-distance launches that ran on the tensor cores
+ * [22] key lines (32 keys) the nucleotide selection opened, first pass */
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset);
 
 /* ---- host side of SURVEY.md section 8 (f1) / (f3) in native code (no CUDA kernel involved) ---- */
