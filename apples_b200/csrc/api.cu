@@ -69,11 +69,13 @@ struct apples_ctx {
     bool bytes_ready = false;     // ref_bytes_p / rep_bytes_p hold the reference
     DevBuf ref_bytes_p, rep_bytes_p, q_bytes_p, q_rowflag, keys_w;
     double n_slow = 0;            // queries that went through the fallback
-    // representative-count kernel: 1 = tcgen05 kind::i8 tensor-core kernel (dense_tc.cu, default), 0 = integer-pipe LOP3/POPC
-    // kernel (distance.cu; also taken automatically beyond 33 816 columns)
+    // representative-count kernel: 1 = tensor cores (dense_tc.cu, default): the block-scaled fp4 kernel up to
+    // dense_fp4_max_sites() columns, the kind::i8 kernel beyond it; 0 = integer-pipe LOP3/POPC kernel (distance.cu; also
+    // taken automatically beyond 33 816 columns)
     int dense_mode = 1;
-    double n_tc_launch = 0;
+    double n_tc_launch = 0, n_fp4_launch = 0;
     bool tc_ready = false;        // reps_img holds the representatives' operand images
+    bool tc_fp4 = false;          // ... for the fp4 kernel (else for the kind::i8 kernel)
     int tc_nw = 0, tc_rep_pad = 0;
     DevBuf reps_img, q_img;
     bool refs_wm_ready = false;
@@ -311,7 +313,11 @@ int set_geometry(apples_ctx* ctx, int kind, int L, int n_ref, const int32_t* ref
     ctx->W = apples_words_per_row(L);
     ctx->Wp = round_up(ctx->W, DT_WC);
     ctx->Lp = apples_aa_row_bytes(L);
-    ctx->rep_pad = round_up(n_rep, ctx->dense_mode == 1 ? 256 : DT_TR);
+    // the key row (ldk = rep_pad) covers the representative tiles of the count kernel and stays a multiple of DT_TR
+    if (ctx->dense_mode == 1 && L <= dense_fp4_max_sites())
+        ctx->rep_pad = round_up(round_up(n_rep, dense_fp4_tile_rows(1)), DT_TR);
+    else
+        ctx->rep_pad = round_up(n_rep, ctx->dense_mode == 1 ? 256 : DT_TR);
     ctx->ref_pad = round_up(n_ref, DT_TR);
     const size_t row = query_row_bytes(ctx);
     if (ensure(ctx, ctx->refs_rm, (size_t)n_ref * row) || ensure(ctx, ctx->reps_rm, (size_t)n_rep * row) ||
@@ -337,9 +343,17 @@ int prepare_operands(apples_ctx* ctx, cudaStream_t s) {
     // operand images of the representatives for the tensor-core kernel
     if (ctx->dense_mode != 1 || ctx->L > dense_tc_max_sites()) return 0;
     ctx->tc_nw = (ctx->L + 31) / 32;
-    ctx->tc_rep_pad = round_up(ctx->n_rep, dense_tc_tile_rows());
-    if (ensure(ctx, ctx->reps_img, dense_tc_image_bytes(ctx->tc_rep_pad, ctx->tc_nw))) return -1;
-    launch_tc_image((const uint32_t*)ctx->reps_rm.p, ctx->n_rep, ctx->W, ctx->tc_nw, ctx->tc_rep_pad, 127, ctx->reps_img.p, s);
+    ctx->tc_fp4 = ctx->L <= dense_fp4_max_sites();
+    if (ctx->tc_fp4) {
+        ctx->tc_rep_pad = round_up(ctx->n_rep, dense_fp4_tile_rows(1));
+        if (ensure(ctx, ctx->reps_img, dense_fp4_image_bytes(ctx->tc_rep_pad, ctx->tc_nw))) return -1;
+        launch_fp4_image((const uint32_t*)ctx->reps_rm.p, ctx->n_rep, ctx->W, ctx->tc_nw, ctx->tc_rep_pad, dense_fp4_tile_rows(1),
+                         ctx->reps_img.p, s);
+    } else {
+        ctx->tc_rep_pad = round_up(ctx->n_rep, dense_tc_tile_rows());
+        if (ensure(ctx, ctx->reps_img, dense_tc_image_bytes(ctx->tc_rep_pad, ctx->tc_nw))) return -1;
+        launch_tc_image((const uint32_t*)ctx->reps_rm.p, ctx->n_rep, ctx->W, ctx->tc_nw, ctx->tc_rep_pad, 127, ctx->reps_img.p, s);
+    }
     CK(cudaGetLastError());
     ctx->tc_ready = true;
     return 0;
@@ -512,7 +526,9 @@ struct MacroBatch {
     int allocate() {
         if (ensure(ctx, ctx->keys, (size_t)(use_tc ? round_up(QB, 256) : QB) * ldk * key_bytes)) return -1;
         if (sel_kind == SEL_NUC && ensure(ctx, ctx->kmin, (size_t)(use_tc ? round_up(QB, 256) : QB) * (ldk / 32) * 4)) return -1;
-        if (use_tc && ensure(ctx, ctx->q_img, dense_tc_image_bytes(round_up(QB, 256), ctx->tc_nw))) return -1;
+        if (use_tc && ensure(ctx, ctx->q_img, ctx->tc_fp4 ? dense_fp4_image_bytes(round_up(QB, dense_fp4_tile_rows(0)), ctx->tc_nw)
+                                                          : dense_tc_image_bytes(round_up(QB, 256), ctx->tc_nw)))
+            return -1;
         if (io.h_bytes) {
             if (ensure(ctx, ctx->q_bytes, (size_t)QB * io.byte_stride) || ensure(ctx, ctx->bad_flag, 4)) return -1;
             if (two_bufs && ensure(ctx, ctx->q_bytes2, (size_t)QB * io.byte_stride)) return -1;
@@ -773,6 +789,23 @@ struct MacroBatch {
             ctx->n_dense_launch += 1;
             ctx->n_pairs += (double)nb * ctx->n_rep;
             ctx->n_slow += nb;
+        } else if (sel_kind == SEL_NUC && use_tc && ctx->tc_fp4) {
+            const int q_pad = round_up(nb, dense_fp4_tile_rows(0));
+            {
+                Span sp(ctx, T_TRANSPOSE, st);
+                launch_fp4_image((const uint32_t*)d_q, nb, ctx->W, ctx->tc_nw, q_pad, dense_fp4_tile_rows(0), ctx->q_img.p, st);
+                ctx->n_launch += 1;
+            }
+            {
+                Span sp(ctx, T_DENSE, st);
+                launch_dense_fp4(ctx->q_img.p, q_pad, ctx->reps_img.p, ctx->tc_rep_pad, ctx->tc_nw, (uint32_t*)ctx->keys.p, ldk,
+                                 (uint32_t*)ctx->kmin.p, sa.gate.vmin, ctx->num_sms, st);
+                ctx->n_launch += 1;
+                ctx->n_dense_launch += 1;
+                ctx->n_tc_launch += 1;
+                ctx->n_fp4_launch += 1;
+            }
+            ctx->n_pairs += (double)nb * ctx->n_rep;
         } else if (sel_kind == SEL_NUC && use_tc) {
             const int q_pad = round_up(nb, 256);
             {
@@ -1711,17 +1744,18 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
 
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset) {
     if (!ctx || !out) return -1;
-    double v[23] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
+    double v[24] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
                     ctx->t_ms[T_D2H], ctx->n_launch, ctx->n_dense_launch, ctx->n_pairs, ctx->n_obs, ctx->n_valid,
                     ctx->n_over, ctx->max_K, ctx->max_V, ctx->dense_mhz, ctx->n_place_class[0], ctx->n_place_class[1],
-                    ctx->n_place_class[2], ctx->n_place_class[3], ctx->n_place_class[4], ctx->n_slow, ctx->n_tc_launch, ctx->n_lines};
-    for (int i = 0; i < n && i < 23; ++i) out[i] = v[i];
+                    ctx->n_place_class[2], ctx->n_place_class[3], ctx->n_place_class[4], ctx->n_slow, ctx->n_tc_launch, ctx->n_lines,
+                    ctx->n_fp4_launch};
+    for (int i = 0; i < n && i < 24; ++i) out[i] = v[i];
     if (reset) {
         for (int i = 0; i < T_NSTAGE; ++i) ctx->t_ms[i] = 0;
         ctx->n_launch = ctx->n_dense_launch = ctx->n_pairs = ctx->n_lines = ctx->n_obs = ctx->n_valid = ctx->n_over = ctx->max_K = ctx->max_V = 0;
         for (int c = 0; c < PLACE_NCLASS; ++c) ctx->n_place_class[c] = 0;
         ctx->n_slow = 0;
-        ctx->n_tc_launch = 0;
+        ctx->n_tc_launch = ctx->n_fp4_launch = 0;
     }
     return 0;
 }

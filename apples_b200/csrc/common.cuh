@@ -243,6 +243,13 @@ size_t dense_tc_image_bytes(int rows_pad, int n_w);
 void launch_tc_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int vw, void* out, cudaStream_t s);
 void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
                      uint32_t* kmin, int vmin, int num_sms, cudaStream_t s);
+// block-scaled fp4 count kernel (dense_tc.cu): tiles of 128 queries (side 0) x 224 representatives (side 1)
+int dense_fp4_max_sites();
+int dense_fp4_tile_rows(int side);
+size_t dense_fp4_image_bytes(int rows_pad, int n_w);
+void launch_fp4_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int tile_rows, void* out, cudaStream_t s);
+void launch_dense_fp4(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
+                      uint32_t* kmin, int vmin, int num_sms, cudaStream_t s);
 cudaError_t launch_pack(int kind, const uint8_t* bytes, int64_t row_stride, int n, int L, void* out, int* bad, cudaStream_t s,
                         int* row_flag = nullptr);
 cudaError_t launch_repitch_bytes(const uint8_t* src, int64_t src_stride, int n, int L, int Lp, uint8_t* dst, cudaStream_t s);

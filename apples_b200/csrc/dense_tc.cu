@@ -1,6 +1,8 @@
-// Kernel (a), default for nucleotide alignments: the query x representative count stage (apples/distance.py:733-737 as
-// called from apples/Reference.py:138-142) on the 5th-generation tensor cores (tcgen05.mma kind::i8, accumulators in TMEM),
+// Kernel (a1): the query x representative count stage (apples/distance.py:733-737 as called from
+// apples/Reference.py:138-142) on the 5th-generation tensor cores (tcgen05.mma kind::i8, accumulators in TMEM),
 // bit-identical to the LOP3/POPC kernel of distance.cu (which stays selectable: apples_ctx_set_dense_mode(ctx, 0)).
+// The block-scaled fp4 kernel at the end of this file (kernel (a), the default) takes alignments up to FP4_MAX_L sites;
+// this one takes the rest up to TC_MAX_L.
 //
 // BASELINE.json's north star says "no tensor cores are used, since nothing here is a dense contraction".  The mismatch
 // count IS a contraction once the alphabet is embedded in a regular simplex: with
@@ -147,22 +149,25 @@ struct TcArgs {
     int sq, sr;             // super-tile shape (query tiles x representative tiles) of the L2-friendly tile order
 };
 
-// tile index -> (query tile, representative tile): super-tiles of sq x sr tiles, so that the ~148 CTAs of a wave share a
-// few operand images in L2 instead of streaming all representatives for every pair of query tiles
-__device__ __forceinline__ void tc_tile(const TcArgs& a, int t, int& qt, int& rt) {
-    const int n_qt = a.q_pad / TC_TM, n_rt = a.r_pad / TC_TN;
-    const int per_band = a.sq * n_rt;              // tiles of a band of sq query tiles
+// tile index -> (query tile, representative tile) of an n_qt x n_rt tile grid: super-tiles of sq x sr tiles, so that the
+// ~148 CTAs of a wave share a few operand images in L2 instead of streaming all representatives for every pair of query
+// tiles
+__device__ __forceinline__ void super_tile(int n_qt, int n_rt, int sq, int sr, int t, int& qt, int& rt) {
+    const int per_band = sq * n_rt;                // tiles of a band of sq query tiles
     const int band = t / per_band, in_band = t % per_band;
-    const int q0 = band * a.sq;
-    const int qh = min(a.sq, n_qt - q0);           // the last band may be thinner
-    const int col = in_band / (qh * a.sr);         // super-tile column inside the band
-    const int rem = in_band % (qh * a.sr);
-    const int r0 = col * a.sr;
-    const int rw = min(a.sr, n_rt - r0);
+    const int q0 = band * sq;
+    const int qh = min(sq, n_qt - q0);             // the last band may be thinner
+    const int col = in_band / (qh * sr);           // super-tile column inside the band
+    const int rem = in_band % (qh * sr);
+    const int r0 = col * sr;
+    const int rw = min(sr, n_rt - r0);
     // inside a (qh x rw) super-tile: row-major over its tiles; in_band was laid out with full-width columns of qh * sr tiles
     // except the last column, which holds qh * rw tiles
     qt = q0 + rem / rw;
     rt = r0 + rem % rw;
+}
+__device__ __forceinline__ void tc_tile(const TcArgs& a, int t, int& qt, int& rt) {
+    super_tile(a.q_pad / TC_TM, a.r_pad / TC_TN, a.sq, a.sr, t, qt, rt);
 }
 
 __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a) {
@@ -314,11 +319,299 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a)
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
 }
 
+// ===============================================================================================================
+// Kernel (a) on block-scaled fp4 (tcgen05.mma kind::mxf4, all scale factors 1.0): the default for alignments of up to
+// FP4_MAX_L sites.  The kind::i8 kernel above needs 4 operand bytes per site because one s32 accumulator carries both
+// counts through the weight 63503; fp4 cannot hold those weights, so the counts go to TWO fp32 accumulators instead,
+// and each operand element goes to exactly one of them:
+//     D1 = sum of the three +-1 simplex components   = 3 match - mismatch   (in [-L, 3L])
+//     D2 = sum of the validity component (1 or 0)    = match + mismatch     (in [0, L])
+// Both are small integers, exact in fp32 (tests/test_gpu_count_fp4.py checks the whole range on the device), and
+//     match = (D1 + D2) / 4,   mismatch = D2 - match.
+// A site is 4 e2m1 elements = 2 bytes of K instead of 4.
+//
+// Kernel: the same persistent structure as dense_tc_kernel (producer warp, MMA warp, 8 epilogue warps, super-tile order,
+// streaming key stores, line minima).  CTA tile 128 queries x 224 representatives: D1 in TMEM columns 0..223, D2 in
+// 256..479, the constant scale factors in 480..511.  A stage is 64 sites = 128 bytes of K per row (A 16 KB + B 28 KB),
+// 4 stages.  Per stage the MMA warp issues 4 MMAs of K = 64: the x, y and z slices into D1, the validity slice into D2.
+// Operand images are K-major, no swizzle, in 128-byte core matrices as above: [k16 = 8][row block = R / 8][8 rows][16 B]
+// with R = 128 or 224 rows, so LBO = 16 R bytes; the 16-byte piece k16 = 2 * component + (word & 1) holds the 32 sites
+// of one plane word, site s in nibble s.  The MMA sums over all of K, so only the SAME order on both sides matters.
+// ===============================================================================================================
+#ifndef FP4_MAX_L_V
+#define FP4_MAX_L_V 33816
+#endif
+constexpr int FP4_MAX_L = FP4_MAX_L_V;      // longest alignment of the fp4 kernel (build-time knob for measurements)
+constexpr int F4_TM = 128;                  // query rows per CTA tile
+constexpr int F4_TN = 224;                  // representative rows per CTA tile (whole 32-key lines: 7)
+constexpr int F4_KS = 128;                  // K bytes per row and stage = 64 sites x 4 components x 4 bits
+constexpr int F4_STAGES = 4;
+constexpr int F4_A = F4_TM * F4_KS;         // 16 KB
+constexpr int F4_B = F4_TN * F4_KS;         // 28 KB
+constexpr int F4_STAGE = F4_A + F4_B;
+constexpr int F4_SMEM = F4_STAGES * F4_STAGE + 1024 + 256 + TC_EPI_WARPS * TC_XPOSE;
+constexpr uint32_t F4_D2 = 256, F4_SFA = 480, F4_SFB = 496;   // TMEM columns of D2 and of the scale factors
+// kind::mxf4 (UMMA::InstrDescriptorBlockScaled): A = B = E2M1 (1) at bits 7 and 10, both K-major, N >> 3 at bit 17,
+// scale format UE8M0 at bit 23, M >> 4 at bit 24, scale-factor ids 0, K = 64
+constexpr uint32_t F4_IDESC = (1u << 7) | (1u << 10) | ((uint32_t)(F4_TN >> 3) << 17) | (1u << 23) | ((uint32_t)(F4_TM >> 4) << 24);
+constexpr uint32_t F4_ONES = 0x7f7f7f7fu;   // four UE8M0 scale factors of 2^0
+
+__device__ __forceinline__ void f4_mma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t sfa, uint32_t sfb,
+                                       uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %6, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t}"
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(F4_IDESC), "r"(sfa), "r"(sfb), "r"(accumulate)
+        : "memory");
+}
+
+// 8 bits -> bit i at bit 4 i
+__device__ __forceinline__ uint32_t f4_spread(uint32_t b) {
+    b = (b | (b << 12)) & 0x000f000fu;
+    b = (b | (b << 6)) & 0x03030303u;
+    return (b | (b << 3)) & 0x11111111u;
+}
+// the 32 sites of one component as e2m1 nibbles: +1 = 0x2, -1 = 0xa (neg = sign bits), 0 where `valid` is clear
+__device__ __forceinline__ uint4 f4_nibbles(uint32_t valid, uint32_t neg) {
+    uint32_t o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) o[j] = (f4_spread((valid >> (8 * j)) & 0xffu) << 1) | (f4_spread((neg >> (8 * j)) & 0xffu) << 3);
+    return make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// fp4 operand images: bit-planes [rows][3][W] -> [rows_pad / R][n_c][R * 128 bytes], n_c = ceil(n_w / 2) chunks of 64
+// sites (a missing odd word is all gaps).  One thread per (row, word): a warp takes 32 rows of one word, so each of its
+// four 16-byte stores per thread covers 512 contiguous bytes; the 8 warps of a block take 8 consecutive words of the same
+// rows, which share the 32-byte sectors of the plane reads.  The validity component is 1 at every valid site on both sides.
+__global__ void __launch_bounds__(256) fp4_image_kernel(const uint32_t* __restrict__ planes, int rows, int W, int n_w, int R,
+                                                        uint4* __restrict__ out) {
+    const int n_c = (n_w + 1) / 2;
+    const int r = blockIdx.y * 32 + (threadIdx.x & 31);
+    const int w = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (w >= 2 * n_c) return;
+    uint32_t lo = 0, hi = 0, va = 0;
+    if (r < rows && w < n_w) {
+        const uint32_t* p = planes + (size_t)r * 3 * W + w;
+        lo = p[0];
+        hi = p[W];
+        va = p[2 * W];
+    }
+    const int rr = r % R;
+    uint4* img = out + ((size_t)(r / R) * n_c + (w >> 1)) * (R * 8) + (rr >> 3) * 8 + (rr & 7);
+    // A(0)=(+,+,+) C(1)=(+,-,-) G(2)=(-,+,-) T(3)=(-,-,+), code = lo | hi << 1 (as tc_image_kernel)
+    const int k = w & 1;
+    img[(0 + k) * R] = f4_nibbles(va, hi & va);          // k16 piece = R / 8 core matrices = R * 8 uint4
+    img[(2 + k) * R] = f4_nibbles(va, lo & va);
+    img[(4 + k) * R] = f4_nibbles(va, (lo ^ hi) & va);
+    img[(6 + k) * R] = f4_nibbles(va, 0u);
+}
+
+__global__ void __launch_bounds__(TC_THREADS, 1) dense_fp4_kernel(const TcArgs a) {   // a.n_w = chunks of 64 sites
+    extern __shared__ unsigned char tc_smem_raw[];
+    unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~(uintptr_t)1023);
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + F4_STAGES * F4_STAGE);
+    uint64_t* empty = full + F4_STAGES;
+    uint64_t* tfull = empty + F4_STAGES;
+    uint64_t* tempty = tfull + 1;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 1);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int n_qt = a.q_pad / F4_TM, n_rt = a.r_pad / F4_TN;
+    const int n_tiles = n_qt * n_rt;
+
+    if (tid == 0) {
+        for (int s = 0; s < F4_STAGES; ++s) {
+            tc_mbar_init(&full[s], 1);
+            tc_mbar_init(&empty[s], 1);
+        }
+        tc_mbar_init(tfull, 1);
+        tc_mbar_init(tempty, TC_EPI_WARPS);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(tc_smem_u32(tmem_slot)) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const uint32_t tmem = *tmem_slot;
+    // scale factors: 1.0 in every byte of columns 480..511 of all 128 lanes, by warps 2..5 (one per lane quarter)
+    if (warp >= 2 && warp < 6) {
+        const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + F4_SFA;
+        const uint32_t o = F4_ONES;
+        asm volatile(
+            "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+            "{%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, "
+            "%1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1, %1};" ::"r"(taddr), "r"(o)
+            : "memory");
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+
+    if (warp == 0) {
+        // ===== producer =====
+        if (lane == 0) {
+            uint32_t it = 0;
+            for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+                int qt, rt;
+                super_tile(n_qt, n_rt, a.sq, a.sr, t, qt, rt);
+                for (int c = 0; c < a.n_w; ++c, ++it) {
+                    const int s = it % F4_STAGES;
+                    tc_mbar_wait(&empty[s], ((it / F4_STAGES) & 1) ^ 1);
+                    tc_mbar_expect_tx(&full[s], F4_STAGE);
+                    unsigned char* sa = smem + (size_t)s * F4_STAGE;
+                    tc_bulk_g2s(sa, a.a_img + ((size_t)qt * a.n_w + c) * F4_A, F4_A, &full[s]);
+                    tc_bulk_g2s(sa + F4_A, a.b_img + ((size_t)rt * a.n_w + c) * F4_B, F4_B, &full[s]);
+                }
+            }
+        }
+    } else if (warp == 1) {
+        // ===== MMA issuer =====
+        if (lane == 0) {
+            const uint32_t sfa = tmem + F4_SFA, sfb = tmem + F4_SFB;
+            uint32_t it = 0, tl = 0;
+            for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++tl) {
+                tc_mbar_wait(tempty, (tl & 1) ^ 1);
+                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                for (int c = 0; c < a.n_w; ++c, ++it) {
+                    const int s = it % F4_STAGES;
+                    tc_mbar_wait(&full[s], (it / F4_STAGES) & 1);
+                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    const uint32_t sa = tc_smem_u32(smem + (size_t)s * F4_STAGE), sb = sa + F4_A;
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {   // components x, y, z into D1, validity into D2
+                        const uint64_t ad = tc_desc(sa + 2 * k * (F4_TM * 16), F4_TM * 16, 128);
+                        const uint64_t bd = tc_desc(sb + 2 * k * (F4_TN * 16), F4_TN * 16, 128);
+                        if (k < 3)
+                            f4_mma(tmem, ad, bd, sfa, sfb, (c > 0 || k > 0) ? 1u : 0u);
+                        else
+                            f4_mma(tmem + F4_D2, ad, bd, sfa, sfb, c > 0 ? 1u : 0u);
+                    }
+                    tc_commit(&empty[s]);
+                }
+                tc_commit(tfull);
+            }
+        }
+    } else {
+        // ===== epilogue: two warps per TMEM lane quarter; g = 0 takes the lines 0..3 of the tile row, g = 1 the lines 4..6 =====
+        const int quarter = warp & 3, g = (warp - 2) >> 2;
+        const int c0 = g * 128, c1 = g ? F4_TN : 128;
+        uint32_t* xp = reinterpret_cast<uint32_t*>(smem + F4_STAGES * F4_STAGE + 256) + (size_t)(warp - 2) * (TC_XPOSE / 4);
+        uint32_t tl = 0;
+        for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++tl) {
+            int qt, rt;
+            super_tile(n_qt, n_rt, a.sq, a.sr, t, qt, rt);
+            tc_mbar_wait(tfull, tl & 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const int row0 = qt * F4_TM + quarter * 32;
+            uint32_t lm0 = LINE_NONE, lm1 = LINE_NONE, lm2 = LINE_NONE, lm3 = LINE_NONE;
+#pragma unroll 1
+            for (int c = c0; c < c1; c += 32) {
+                uint32_t d1[32], d2[32];
+                const uint32_t taddr = tmem + ((uint32_t)(quarter * 32) << 16) + (uint32_t)c;
+                asm volatile(
+                    "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+                    "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+                    "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+                    : "=r"(d1[0]), "=r"(d1[1]), "=r"(d1[2]), "=r"(d1[3]), "=r"(d1[4]), "=r"(d1[5]), "=r"(d1[6]), "=r"(d1[7]),
+                      "=r"(d1[8]), "=r"(d1[9]), "=r"(d1[10]), "=r"(d1[11]), "=r"(d1[12]), "=r"(d1[13]), "=r"(d1[14]), "=r"(d1[15]),
+                      "=r"(d1[16]), "=r"(d1[17]), "=r"(d1[18]), "=r"(d1[19]), "=r"(d1[20]), "=r"(d1[21]), "=r"(d1[22]), "=r"(d1[23]),
+                      "=r"(d1[24]), "=r"(d1[25]), "=r"(d1[26]), "=r"(d1[27]), "=r"(d1[28]), "=r"(d1[29]), "=r"(d1[30]), "=r"(d1[31])
+                    : "r"(taddr)
+                    : "memory");
+                asm volatile(
+                    "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+                    "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+                    "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+                    : "=r"(d2[0]), "=r"(d2[1]), "=r"(d2[2]), "=r"(d2[3]), "=r"(d2[4]), "=r"(d2[5]), "=r"(d2[6]), "=r"(d2[7]),
+                      "=r"(d2[8]), "=r"(d2[9]), "=r"(d2[10]), "=r"(d2[11]), "=r"(d2[12]), "=r"(d2[13]), "=r"(d2[14]), "=r"(d2[15]),
+                      "=r"(d2[16]), "=r"(d2[17]), "=r"(d2[18]), "=r"(d2[19]), "=r"(d2[20]), "=r"(d2[21]), "=r"(d2[22]), "=r"(d2[23]),
+                      "=r"(d2[24]), "=r"(d2[25]), "=r"(d2[26]), "=r"(d2[27]), "=r"(d2[28]), "=r"(d2[29]), "=r"(d2[30]), "=r"(d2[31])
+                    : "r"(taddr + F4_D2)
+                    : "memory");
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                // decode and line minimum as in dense_tc_kernel.  fp32 -> integer by the 1.5 * 2^23 shift (exact for
+                // |x| < 2^22): D1 + D2 = 4 match and D2 = valid are integers in [0, 4 L]
+                uint32_t bmi = 1u, bma = 0u;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) {
+                    const float f1 = __int_as_float((int)d1[j]), f2 = __int_as_float((int)d2[j]);
+                    const uint32_t m4 = (uint32_t)__float_as_int((f1 + f2) + 12582912.0f) - 0x4b400000u;
+                    const uint32_t valid = (uint32_t)__float_as_int(f2 + 12582912.0f) - 0x4b400000u;
+                    const uint32_t match = m4 >> 2;
+                    const uint32_t mism = valid - match;
+                    xp[lane * 33 + j] = mism | (valid << 16);
+                    const bool lower = valid >= a.vmin1 && mism * bma < bmi * match;
+                    bmi = lower ? mism : bmi;
+                    bma = lower ? match : bma;
+                }
+                lm0 = lm1;
+                lm1 = lm2;
+                lm2 = lm3;
+                lm3 = (bmi < 3u * bma) ? (bmi | ((bmi + bma) << 16)) : LINE_NONE;
+                __syncwarp();
+#pragma unroll
+                for (int r0 = 0; r0 < 32; r0 += 4) {
+                    const int rr = r0 + (lane >> 3), cc = (lane & 7) * 4;
+                    const uint4 o = make_uint4(xp[rr * 33 + cc], xp[rr * 33 + cc + 1], xp[rr * 33 + cc + 2], xp[rr * 33 + cc + 3]);
+                    __stcs(reinterpret_cast<uint4*>(a.keys + (size_t)(row0 + rr) * a.ldk + (size_t)rt * F4_TN + c + cc), o);
+                }
+                __syncwarp();
+            }
+            // the warp's lines of its row: lm0..lm3 = lines 0..3 (g = 0), lm1..lm3 = lines 4..6 (g = 1)
+            uint32_t* mrow = a.kmin + (size_t)(row0 + lane) * (a.ldk / 32) + (size_t)rt * (F4_TN / 32) + 3 * g;
+            if (g == 0) __stcs(mrow, lm0);
+            __stcs(mrow + 1, lm1);
+            __stcs(mrow + 2, lm2);
+            __stcs(mrow + 3, lm3);
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            __syncwarp();
+            if (lane == 0) tc_mbar_arrive(tempty);
+        }
+    }
+    __syncthreads();
+    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+}
+
 // function attributes are per device: called by apples_ctx_create on the context's device
 cudaError_t dense_tc_configure() {
     cudaError_t e = cudaFuncSetAttribute(tc_image_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TCI_SMEM);
     if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(dense_fp4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F4_SMEM);
+    if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(dense_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+}
+
+int dense_fp4_max_sites() { return FP4_MAX_L < TC_MAX_L ? FP4_MAX_L : TC_MAX_L; }
+int dense_fp4_tile_rows(int side) { return side ? F4_TN : F4_TM; }
+size_t dense_fp4_image_bytes(int rows_pad, int n_w) { return (size_t)rows_pad * ((n_w + 1) / 2) * F4_KS; }
+
+void launch_fp4_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int tile_rows, void* out, cudaStream_t s) {
+    if (rows_pad <= 0 || n_w <= 0) return;
+    const int n_c = (n_w + 1) / 2;
+    dim3 grid((2 * n_c + 7) / 8, rows_pad / 32);
+    fp4_image_kernel<<<grid, 256, 0, s>>>(planes, rows, W, n_w, tile_rows, (uint4*)out);
+}
+
+void launch_dense_fp4(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
+                      uint32_t* kmin, int vmin, int num_sms, cudaStream_t s) {
+    TcArgs a;
+    a.a_img = (const uint8_t*)a_img;
+    a.b_img = (const uint8_t*)b_img;
+    a.q_pad = q_pad;
+    a.r_pad = r_pad;
+    a.n_w = (n_w + 1) / 2;
+    a.keys = keys;
+    a.ldk = ldk;
+    a.kmin = kmin;
+    a.vmin1 = (uint32_t)(vmin > 1 ? vmin : 1);
+    a.sq = 12;
+    a.sr = 12;
+    const int tiles = (q_pad / F4_TM) * (r_pad / F4_TN);
+    dense_fp4_kernel<<<tiles < num_sms ? tiles : num_sms, TC_THREADS, F4_SMEM, s>>>(a);
 }
 
 int dense_tc_max_sites() { return TC_MAX_L; }

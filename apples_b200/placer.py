@@ -221,12 +221,13 @@ class GpuPlacer:
         return K, V, ov
 
     def timings(self, reset=False):
-        v = np.zeros(23, np.float64)
-        self.lib.apples_get_timings(self.h, _lib.ptr(v), 23, 1 if reset else 0)
+        v = np.zeros(24, np.float64)
+        self.lib.apples_get_timings(self.h, _lib.ptr(v), 24, 1 if reset else 0)
         keys = ['h2d_ms', 'transpose_ms', 'rep_distance_ms', 'selection_ms', 'placement_ms', 'd2h_ms', 'launches',
                 'rep_distance_launches', 'pairs', 'observed', 'valid_nodes', 'overflow_queries', 'max_observed',
                 'max_valid_nodes', 'rep_distance_sm_mhz', 'placed_smem64', 'placed_smem128', 'placed_smem256',
-                'placed_smem512', 'placed_block', 'fallback_queries', 'tensor_core_launches', 'key_lines_read']
+                'placed_smem512', 'placed_block', 'fallback_queries', 'tensor_core_launches', 'key_lines_read',
+                'fp4_launches']
         return dict(zip(keys, v.tolist()))
 
     # ------------------------------------------------------------------------------------------------ parity exports

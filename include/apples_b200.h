@@ -80,10 +80,12 @@ void* apples_ctx_stream(apples_ctx* ctx);
 int apples_ctx_set_limits(apples_ctx* ctx, int64_t max_subbatch, int64_t scratch_bytes, int32_t slot_cap);
 
 /* Which kernel computes the query x representative mismatch / overlap counts of nucleotide alignments.
- * 1 (default) = the tcgen05 kind::i8 tensor-core kernel (dense_tc.cu): the two counts of distance.py:733-737 as ONE int8 dot
- * product per pair (simplex embedding of A,C,G,T; exact s32 accumulation in TMEM); 0 = the integer-pipe LOP3/POPC kernel of
- * the north star (distance.cu).  Both give bit-identical 32-bit keys.  Call before apples_set_reference*.  Alignments the
- * tensor-core kernel does not cover (more than 33 816 columns) use the integer-pipe kernel automatically. */
+ * 1 (default) = the tcgen05 tensor-core kernels (dense_tc.cu): the block-scaled fp4 kernel (kind::mxf4; simplex embedding
+ * of A,C,G,T into one fp32 accumulator, validity into a second, both exact) up to its length limit, the kind::i8 kernel
+ * (the two counts of distance.py:733-737 as ONE int8 dot product per pair, exact s32 accumulation in TMEM) beyond it;
+ * 0 = the integer-pipe LOP3/POPC kernel of the north star (distance.cu).  All give bit-identical 32-bit keys.  Call before
+ * apples_set_reference*.  Alignments the tensor-core kernels do not cover (more than 33 816 columns) use the
+ * integer-pipe kernel automatically. */
 int apples_ctx_set_dense_mode(apples_ctx* ctx, int32_t mode);
 
 /* Backbone tree as flat arrays over the M nodes (replaces the treeswift node graph prepared by
@@ -198,7 +200,8 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
  * [15..19] queries placed by the shared-memory placement launches of 64 / 128 / 256 / 512 node slots and by the
  * block-per-query launch (global scratch)  [20] queries that went through the byte-compare fallback
  * [21] representative-distance launches that ran on the tensor cores
- * [22] key lines (32 keys) the nucleotide selection opened, first pass */
+ * [22] key lines (32 keys) the nucleotide selection opened, first pass
+ * [23] representative-distance launches that ran the block-scaled fp4 tensor-core kernel (counted in [21] too) */
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset);
 
 /* ---- host side of SURVEY.md section 8 (f1) / (f3) in native code (no CUDA kernel involved) ---- */
