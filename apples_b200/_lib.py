@@ -19,12 +19,14 @@ PLACED, ZERO_DIST_LEAF, TOO_FEW_DISTANCES, PLACED_MISPLACEMENT_FLAG = 0, 1, 2, 3
 FLAG_PENDANT_INT0 = 0x100
 FLAG_DEGENERATE = 0x200
 MAX_KEEP = 16            # APPLES_MAX_KEEP: ranked records per query (apples_set_alternatives)
+JC69, K2P = 0, 1         # APPLES_JC69 / APPLES_K2P: nucleotide distance model (apples_ctx_set_model)
+MODELS = {'JC69': JC69, 'K2P': K2P}
 NEWICK_UNSUPPORTED = 1   # apples_newick_*: text outside the native parser's language, use the Python twin
 
 # every symbol the header declares (tests/test_cabi.py checks the library exports exactly these)
 SYMBOLS = [
     'apples_words_per_row', 'apples_aa_row_bytes', 'apples_device_count', 'apples_ctx_create', 'apples_ctx_destroy', 'apples_last_error',
-    'apples_ctx_stream', 'apples_ctx_set_limits', 'apples_ctx_set_dense_mode', 'apples_set_tree', 'apples_set_reference', 'apples_set_matrix_columns', 'apples_place_batch',
+    'apples_ctx_stream', 'apples_ctx_set_limits', 'apples_ctx_set_dense_mode', 'apples_ctx_set_model', 'apples_set_tree', 'apples_set_reference', 'apples_set_matrix_columns', 'apples_place_batch',
     'apples_place_batch_matrix', 'apples_set_reference_bytes', 'apples_place_batch_bytes', 'apples_queries_upload', 'apples_place_resident', 'apples_results_download', 'apples_results_to_device',
     'apples_set_alternatives', 'apples_distance_counts', 'apples_count_keys', 'apples_observed_sets', 'apples_edge_solutions', 'apples_get_timings', 'apples_last_counts',
     'apples_fasta_open', 'apples_fasta_close', 'apples_fasta_count', 'apples_fasta_max_len', 'apples_fasta_stride',
@@ -70,6 +72,7 @@ def load():
     lib.apples_ctx_stream.restype = vp
     lib.apples_ctx_set_limits.argtypes = [vp, i64, i64, i32]
     lib.apples_ctx_set_dense_mode.argtypes = [vp, i32]
+    lib.apples_ctx_set_model.argtypes = [vp, i32]
     lib.apples_set_tree.argtypes = [vp, i32, vp, vp, vp, vp]
     lib.apples_set_reference.argtypes = [vp, C.c_int, i32, i32, vp, vp, i32, vp, vp, vp]
     lib.apples_set_matrix_columns.argtypes = [vp, i32, vp]

@@ -73,7 +73,11 @@ struct apples_ctx {
     // dense_fp4_max_sites() columns, the kind::i8 kernel beyond it; 0 = integer-pipe LOP3/POPC kernel (distance.cu; also
     // taken automatically beyond 33 816 columns)
     int dense_mode = 1;
-    double n_tc_launch = 0, n_fp4_launch = 0;
+    double n_tc_launch = 0, n_fp4_launch = 0, n_k2p_launch = 0;
+    // substitution model: `model` is the setting for the next apples_set_reference*, `k2p` that of the installed reference
+    // (K2P count keys, 128 x 160 count tiles, the SEL_K2P selection)
+    int model = APPLES_JC69;
+    bool k2p = false;
     bool tc_ready = false;        // reps_img holds the representatives' operand images
     bool tc_fp4 = false;          // ... for the fp4 kernel (else for the kind::i8 kernel)
     int tc_nw = 0, tc_rep_pad = 0;
@@ -314,8 +318,9 @@ int set_geometry(apples_ctx* ctx, int kind, int L, int n_ref, const int32_t* ref
     ctx->Wp = round_up(ctx->W, DT_WC);
     ctx->Lp = apples_aa_row_bytes(L);
     // the key row (ldk = rep_pad) covers the representative tiles of the count kernel and stays a multiple of DT_TR
+    ctx->k2p = ctx->model == APPLES_K2P;
     if (ctx->dense_mode == 1 && L <= dense_fp4_max_sites())
-        ctx->rep_pad = round_up(round_up(n_rep, dense_fp4_tile_rows(1)), DT_TR);
+        ctx->rep_pad = round_up(round_up(n_rep, dense_fp4_tile_rows(1, ctx->k2p)), DT_TR);
     else
         ctx->rep_pad = round_up(n_rep, ctx->dense_mode == 1 ? 256 : DT_TR);
     ctx->ref_pad = round_up(n_ref, DT_TR);
@@ -324,6 +329,16 @@ int set_geometry(apples_ctx* ctx, int kind, int L, int n_ref, const int32_t* ref
         ensure(ctx, ctx->ref_node, (size_t)n_ref * 4) || ensure(ctx, ctx->goff, (size_t)(n_rep + 1) * 4) ||
         ensure(ctx, ctx->gmem, (size_t)std::max(n_mem, 1) * 4))
         return -1;
+    return 0;
+}
+
+// what the K2P model needs of a reference (apples_ctx_set_model), checked before it is installed
+int check_model(apples_ctx* ctx, const char* who, int kind, int L) {
+    if (ctx->model != APPLES_K2P) return 0;
+    if (kind != APPLES_NUC) return fail(ctx, "%s: the K2P model needs nucleotide sequences", who);
+    if (ctx->dense_mode != 1) return fail(ctx, "%s: the K2P model needs the tensor-core count kernel (dense mode 1)", who);
+    if (L > dense_fp4_max_sites())
+        return fail(ctx, "%s: the K2P model takes alignments of at most %d columns, this one has %d", who, dense_fp4_max_sites(), L);
     return 0;
 }
 
@@ -345,10 +360,10 @@ int prepare_operands(apples_ctx* ctx, cudaStream_t s) {
     ctx->tc_nw = (ctx->L + 31) / 32;
     ctx->tc_fp4 = ctx->L <= dense_fp4_max_sites();
     if (ctx->tc_fp4) {
-        ctx->tc_rep_pad = round_up(ctx->n_rep, dense_fp4_tile_rows(1));
+        const int rows = dense_fp4_tile_rows(1, ctx->k2p);
+        ctx->tc_rep_pad = round_up(ctx->n_rep, rows);
         if (ensure(ctx, ctx->reps_img, dense_fp4_image_bytes(ctx->tc_rep_pad, ctx->tc_nw))) return -1;
-        launch_fp4_image((const uint32_t*)ctx->reps_rm.p, ctx->n_rep, ctx->W, ctx->tc_nw, ctx->tc_rep_pad, dense_fp4_tile_rows(1),
-                         ctx->reps_img.p, s);
+        launch_fp4_image((const uint32_t*)ctx->reps_rm.p, ctx->n_rep, ctx->W, ctx->tc_nw, ctx->tc_rep_pad, rows, ctx->reps_img.p, s);
     } else {
         ctx->tc_rep_pad = round_up(ctx->n_rep, dense_tc_tile_rows());
         if (ensure(ctx, ctx->reps_img, dense_tc_image_bytes(ctx->tc_rep_pad, ctx->tc_nw))) return -1;
@@ -454,7 +469,7 @@ struct MacroBatch {
         matrix = io.h_rows != nullptr;
         nuc = !matrix && ctx->kind == APPLES_NUC;
         slow_ctx = nuc && ctx->nuc_slow;
-        sel_kind = matrix ? SEL_MATRIX : (ctx->kind == APPLES_AA ? SEL_AA : (slow_ctx ? SEL_NUCW : SEL_NUC));
+        sel_kind = matrix ? SEL_MATRIX : (ctx->kind == APPLES_AA ? SEL_AA : (slow_ctx ? SEL_NUCW : (ctx->k2p ? SEL_K2P : SEL_NUC)));
         n_units = matrix ? ctx->n_cols : ctx->n_rep;
         ldk = matrix ? ctx->n_cols : ctx->rep_pad;
         key_bytes = (sel_kind == SEL_NUC) ? 4 : 8;
@@ -467,7 +482,8 @@ struct MacroBatch {
         cap_max = next_pow2(std::max(4, matrix ? ctx->n_cols : ctx->n_ref));
         cap = std::min(ctx->slot_cap, cap_max);
         qrow = matrix ? (size_t)ctx->n_cols * 8 : query_row_bytes(ctx);
-        use_tc = sel_kind == SEL_NUC && ctx->tc_ready;
+        // K2P runs on the fp4 kernel whatever apples_ctx_set_dense_mode said after its reference was installed
+        use_tc = sel_kind == SEL_K2P || (sel_kind == SEL_NUC && ctx->tc_ready);
         two_bufs = n > QB;  // more than one sub-batch: stage the next one while this one computes
     }
 
@@ -789,6 +805,24 @@ struct MacroBatch {
             ctx->n_dense_launch += 1;
             ctx->n_pairs += (double)nb * ctx->n_rep;
             ctx->n_slow += nb;
+        } else if (sel_kind == SEL_K2P) {
+            const int q_pad = round_up(nb, dense_fp4_tile_rows(0));
+            {
+                Span sp(ctx, T_TRANSPOSE, st);
+                launch_fp4_image((const uint32_t*)d_q, nb, ctx->W, ctx->tc_nw, q_pad, dense_fp4_tile_rows(0), ctx->q_img.p, st);
+                ctx->n_launch += 1;
+            }
+            {
+                Span sp(ctx, T_DENSE, st);
+                launch_dense_fp4_k2p(ctx->q_img.p, q_pad, ctx->reps_img.p, ctx->tc_rep_pad, ctx->tc_nw,
+                                     (unsigned long long*)ctx->keys.p, ldk, ctx->num_sms, st);
+                ctx->n_launch += 1;
+                ctx->n_dense_launch += 1;
+                ctx->n_tc_launch += 1;
+                ctx->n_fp4_launch += 1;
+                ctx->n_k2p_launch += 1;
+            }
+            ctx->n_pairs += (double)nb * ctx->n_rep;
         } else if (sel_kind == SEL_NUC && use_tc && ctx->tc_fp4) {
             const int q_pad = round_up(nb, dense_fp4_tile_rows(0));
             {
@@ -919,6 +953,10 @@ struct MacroBatch {
                 for (int i = 0; i < n; ++i)
                     if (row_flag[i]) exotic.push_back(i);
             }
+            // K2P is defined on A,C,G,T,- only: no byte-compare fallback
+            if (sel_kind == SEL_K2P && !exotic.empty())
+                return fail(ctx, "query row %lld holds a symbol other than A,C,G,T,-, which the K2P model does not define",
+                            (long long)(base0 + exotic[0]));
         }
         return 0;
     }
@@ -1372,6 +1410,14 @@ int apples_ctx_set_dense_mode(apples_ctx* ctx, int32_t mode) {
     return 0;
 }
 
+int apples_ctx_set_model(apples_ctx* ctx, int32_t model) {
+    if (!ctx) return -1;
+    if (model != APPLES_JC69 && model != APPLES_K2P)
+        return fail(ctx, "apples_ctx_set_model: model must be %d (JC69) or %d (K2P)", APPLES_JC69, APPLES_K2P);
+    ctx->model = model;   // takes effect with the next apples_set_reference*
+    return 0;
+}
+
 int apples_set_tree(apples_ctx* ctx, int32_t M, const int32_t* parent, const double* edge_length, const int32_t* level,
                     const int32_t* first) {
     if (!ctx) return -1;
@@ -1407,7 +1453,9 @@ int apples_set_reference(apples_ctx* ctx, int kind, int32_t L, int32_t n_ref, co
     if ((kind != APPLES_NUC && kind != APPLES_AA) || L <= 0 || n_ref <= 0 || n_rep <= 0 || !packed_refs || !ref_node ||
         !packed_reps || !group_offsets || !group_members)
         return fail(ctx, "apples_set_reference: bad arguments");
-    if (check_reference(ctx, "apples_set_reference", n_ref, ref_node, n_rep, group_offsets, group_members)) return -1;
+    if (check_reference(ctx, "apples_set_reference", n_ref, ref_node, n_rep, group_offsets, group_members) ||
+        check_model(ctx, "apples_set_reference", kind, L))
+        return -1;
     const int n_mem = group_offsets[n_rep];
     if (set_geometry(ctx, kind, L, n_ref, ref_node, n_rep, n_mem)) return -1;
     const size_t row = query_row_bytes(ctx);
@@ -1494,7 +1542,9 @@ int apples_set_reference_bytes(apples_ctx* ctx, int kind, int32_t L, int32_t n_r
     if ((kind != APPLES_NUC && kind != APPLES_AA) || L <= 0 || n_ref <= 0 || n_rep <= 0 || !ref_bytes || row_stride < L ||
         !ref_node || !group_offsets || !group_members)
         return fail(ctx, "apples_set_reference_bytes: bad arguments");
-    if (check_reference(ctx, "apples_set_reference_bytes", n_ref, ref_node, n_rep, group_offsets, group_members)) return -1;
+    if (check_reference(ctx, "apples_set_reference_bytes", n_ref, ref_node, n_rep, group_offsets, group_members) ||
+        check_model(ctx, "apples_set_reference_bytes", kind, L))
+        return -1;
     const int n_mem = group_offsets[n_rep];
     if (set_geometry(ctx, kind, L, n_ref, ref_node, n_rep, n_mem)) return -1;
     cudaStream_t s = ctx->stream;
@@ -1518,6 +1568,11 @@ int apples_set_reference_bytes(apples_ctx* ctx, int kind, int32_t L, int32_t n_r
     // the reference holds bytes other than A,C,G,T,- (ordinary characters for jc69, distance.py:733-737) or is longer
     // than the 16-bit counts allow: keep the byte rows, every query of this context takes the byte-compare fallback
     ctx->nuc_slow = kind == APPLES_NUC && (bad || L > 65535);
+    if (ctx->nuc_slow && ctx->k2p) {
+        ctx->kind = -1;   // the half-installed reference is unusable
+        return fail(ctx, "apples_set_reference_bytes: the reference holds symbols other than A,C,G,T,-, which the K2P model "
+                         "does not define");
+    }
     if (prepare_operands(ctx, s)) return -1;
     if (ctx->nuc_slow) {
         if (ensure(ctx, ctx->ref_bytes_p, (size_t)n_ref * ctx->Lp) || ensure(ctx, ctx->rep_bytes_p, (size_t)n_rep * ctx->Lp))
@@ -1688,7 +1743,7 @@ int apples_count_keys(apples_ctx* ctx, int64_t nq, const void* packed_queries, c
     if (!ctx) return -1;
     if (ctx->kind < 0) return fail(ctx, "apples_set_reference has not been called");
     if (nq <= 0 || !packed_queries || !key_kind || !keys) return fail(ctx, "apples_count_keys: bad arguments");
-    *key_kind = ctx->kind == APPLES_AA ? 2 : (ctx->nuc_slow ? 1 : 0);
+    *key_kind = ctx->kind == APPLES_AA ? 2 : (ctx->nuc_slow ? 1 : (ctx->k2p ? 3 : 0));
     BatchIO io;
     io.h_queries = packed_queries;
     io.h_keys = keys;
@@ -1744,18 +1799,18 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
 
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset) {
     if (!ctx || !out) return -1;
-    double v[24] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
+    double v[25] = {ctx->t_ms[T_H2D], ctx->t_ms[T_TRANSPOSE], ctx->t_ms[T_DENSE], ctx->t_ms[T_SELECT], ctx->t_ms[T_PLACE],
                     ctx->t_ms[T_D2H], ctx->n_launch, ctx->n_dense_launch, ctx->n_pairs, ctx->n_obs, ctx->n_valid,
                     ctx->n_over, ctx->max_K, ctx->max_V, ctx->dense_mhz, ctx->n_place_class[0], ctx->n_place_class[1],
                     ctx->n_place_class[2], ctx->n_place_class[3], ctx->n_place_class[4], ctx->n_slow, ctx->n_tc_launch, ctx->n_lines,
-                    ctx->n_fp4_launch};
-    for (int i = 0; i < n && i < 24; ++i) out[i] = v[i];
+                    ctx->n_fp4_launch, ctx->n_k2p_launch};
+    for (int i = 0; i < n && i < 25; ++i) out[i] = v[i];
     if (reset) {
         for (int i = 0; i < T_NSTAGE; ++i) ctx->t_ms[i] = 0;
         ctx->n_launch = ctx->n_dense_launch = ctx->n_pairs = ctx->n_lines = ctx->n_obs = ctx->n_valid = ctx->n_over = ctx->max_K = ctx->max_V = 0;
         for (int c = 0; c < PLACE_NCLASS; ++c) ctx->n_place_class[c] = 0;
         ctx->n_slow = 0;
-        ctx->n_tc_launch = ctx->n_fp4_launch = 0;
+        ctx->n_tc_launch = ctx->n_fp4_launch = ctx->n_k2p_launch = 0;
     }
     return 0;
 }

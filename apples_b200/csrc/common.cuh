@@ -78,6 +78,20 @@ __device__ __forceinline__ double jc69_from_counts(uint32_t m, uint32_t v, int v
     return -0.75 * log(loc);
 }
 
+// Kimura two-parameter distance from the integer counts: transitions ts, transversions tv, valid sites v (the gate of
+// jc69_from_counts), the fp64 operations of tests/k2p_oracle.py in the same order.  Only for the -fmad=false units: the
+// 0 >= w1 / 0 >= w2 decisions must be the oracle's bit for bit
+__device__ __forceinline__ double k2p_from_counts(uint32_t ts, uint32_t tv, uint32_t v, int vmin) {
+    if (v == 0u || (int)v < vmin) return -1.0;
+    if (ts + tv == 0u) return 0.0;
+    const double P = (double)ts / (double)v;
+    const double Q = (double)tv / (double)v;
+    const double w1 = 1.0 - 2.0 * P - Q;
+    const double w2 = 1.0 - 2.0 * Q;
+    if (0.0 >= w1 || 0.0 >= w2) return -1.0;
+    return -0.5 * log(w1) - 0.25 * log(w2);
+}
+
 // ---- per-line key minima (count stage -> selection).  A line is the 32 keys [32 l, 32 l + 32) of a key row; its minimum
 // is the key of smallest ratio m / v among the keys the selection can use (v >= max(vmin, 1) and 4 m < 3 v, the gate of
 // classify() in select.cu), the smallest column on equal ratios, or LINE_NONE when no key of the line is usable.  A pure
@@ -114,7 +128,7 @@ __device__ __forceinline__ double scoredist_from_sum(double tot, uint32_t v, int
 // ---------------------------------------------------------------------------------------------------------------
 // selection (select.cu) and placement (placement.cu) launch arguments
 // ---------------------------------------------------------------------------------------------------------------
-enum { SEL_NUC = 0, SEL_AA = 1, SEL_MATRIX = 2, SEL_NUCW = 3 };
+enum { SEL_NUC = 0, SEL_AA = 1, SEL_MATRIX = 2, SEL_NUCW = 3, SEL_K2P = 4 };
 
 struct SelectArgs {
     int n;                 // queries in this launch; their key / query rows are rows 0..n-1 of keys_* / q_*
@@ -125,7 +139,7 @@ struct SelectArgs {
     int64_t ldk;           // row stride of the key matrix
     const uint32_t* keys_nuc;  // [nq][ldk] packed (mismatch | valid << 16)
     const uint32_t* kmin;      // SEL_NUC: [nq][ldk / 32] line minima of keys_nuc (LINE_NONE etc., see above)
-    const double* keys_f64;    // [nq][ldk] distances (protein representatives / matrix rows); SEL_NUCW: 64-bit count keys
+    const double* keys_f64;    // [nq][ldk] distances (protein representatives / matrix rows); SEL_NUCW, SEL_K2P: 64-bit count keys
     const int* goff;       // cluster CSR
     const int* gmem;
     const int* ref_node;
@@ -243,13 +257,17 @@ size_t dense_tc_image_bytes(int rows_pad, int n_w);
 void launch_tc_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int vw, void* out, cudaStream_t s);
 void launch_dense_tc(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
                      uint32_t* kmin, int vmin, int num_sms, cudaStream_t s);
-// block-scaled fp4 count kernel (dense_tc.cu): tiles of 128 queries (side 0) x 224 representatives (side 1)
+// block-scaled fp4 count kernel (dense_tc.cu): tiles of 128 queries (side 0) x 224 representatives (side 1), or x 160
+// representatives for the K2P keys (k2p)
 int dense_fp4_max_sites();
-int dense_fp4_tile_rows(int side);
+int dense_fp4_tile_rows(int side, bool k2p = false);
 size_t dense_fp4_image_bytes(int rows_pad, int n_w);
 void launch_fp4_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int tile_rows, void* out, cudaStream_t s);
 void launch_dense_fp4(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, uint32_t* keys, int64_t ldk,
                       uint32_t* kmin, int vmin, int num_sms, cudaStream_t s);
+// K2P keys (ts | tv << 16 | valid << 32) [q_pad][ldk]; b_img built with dense_fp4_tile_rows(1, true) rows per tile
+void launch_dense_fp4_k2p(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, unsigned long long* keys,
+                          int64_t ldk, int num_sms, cudaStream_t s);
 cudaError_t launch_pack(int kind, const uint8_t* bytes, int64_t row_stride, int n, int L, void* out, int* bad, cudaStream_t s,
                         int* row_flag = nullptr);
 cudaError_t launch_repitch_bytes(const uint8_t* src, int64_t src_stride, int n, int L, int Lp, uint8_t* dst, cudaStream_t s);

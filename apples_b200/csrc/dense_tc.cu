@@ -337,6 +337,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_tc_kernel(const TcArgs a)
 // Operand images are K-major, no swizzle, in 128-byte core matrices as above: [k16 = 8][row block = R / 8][8 rows][16 B]
 // with R = 128 or 224 rows, so LBO = 16 R bytes; the 16-byte piece k16 = 2 * component + (word & 1) holds the 32 sites
 // of one plane word, site s in nibble s.  The MMA sums over all of K, so only the SAME order on both sides matters.
+//
+// The K2P instantiation (dense_fp4_kernel<true>) counts transitions and transversions apart.  With code = lo | hi << 1
+// (A=0 C=1 G=2 T=3), lo separates purines from pyrimidines, so over a valid pair the y product is -1 exactly for a
+// transversion, and x x' + z z' is +2 for a match, -2 for a transition and 0 for a transversion.  The y slice goes to a
+// third accumulator D3 instead of D1 (still 4 MMAs per stage, no operand byte added):
+//     D1' = sum (x + z) = 2 (match - ts),   D2 = valid,   D3 = sum y = valid - 2 tv
+// so tv = (D2 - D3) / 2 and ts = (D2 - tv - D1' / 2) / 2, all integers within +-2 L (exact in fp32).  Three 128 x N fp32
+// accumulators and the 32 scale-factor columns fit 512 TMEM columns for N = 160: D1' at 0, D2 at 160, D3 at 320, scale
+// factors at 480 / 496 as above.  The tile is 128 x 160 (5 whole 32-key lines); the epilogue writes 64-bit keys
+// ts | tv << 16 | valid << 32 and folds no line minima.
 // ===============================================================================================================
 #ifndef FP4_MAX_L_V
 #define FP4_MAX_L_V 33816
@@ -351,19 +361,46 @@ constexpr int F4_B = F4_TN * F4_KS;         // 28 KB
 constexpr int F4_STAGE = F4_A + F4_B;
 constexpr int F4_SMEM = F4_STAGES * F4_STAGE + 1024 + 256 + TC_EPI_WARPS * TC_XPOSE;
 constexpr uint32_t F4_D2 = 256, F4_SFA = 480, F4_SFB = 496;   // TMEM columns of D2 and of the scale factors
+// K2P instantiation: 128 x 160 tiles, D2 and D3 at TMEM columns 160 and 320, a 64-bit key transpose block per warp
+constexpr int F4K_TN = 160;
+constexpr int F4K_B = F4K_TN * F4_KS;       // 20 KB
+constexpr int F4K_STAGE = F4_A + F4K_B;
+constexpr int F4K_XPOSE = 32 * 33 * 8;
+constexpr int F4K_SMEM = F4_STAGES * F4K_STAGE + 1024 + 256 + TC_EPI_WARPS * F4K_XPOSE;
+constexpr uint32_t F4K_D2 = 160, F4K_D3 = 320;
 // kind::mxf4 (UMMA::InstrDescriptorBlockScaled): A = B = E2M1 (1) at bits 7 and 10, both K-major, N >> 3 at bit 17,
 // scale format UE8M0 at bit 23, M >> 4 at bit 24, scale-factor ids 0, K = 64
-constexpr uint32_t F4_IDESC = (1u << 7) | (1u << 10) | ((uint32_t)(F4_TN >> 3) << 17) | (1u << 23) | ((uint32_t)(F4_TM >> 4) << 24);
+template <int TN>
+constexpr uint32_t F4_IDESC = (1u << 7) | (1u << 10) | ((uint32_t)(TN >> 3) << 17) | (1u << 23) | ((uint32_t)(F4_TM >> 4) << 24);
 constexpr uint32_t F4_ONES = 0x7f7f7f7fu;   // four UE8M0 scale factors of 2^0
 
+template <int TN>
 __device__ __forceinline__ void f4_mma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t sfa, uint32_t sfb,
                                        uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %6, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(F4_IDESC), "r"(sfa), "r"(sfb), "r"(accumulate)
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(F4_IDESC<TN>), "r"(sfa), "r"(sfb), "r"(accumulate)
         : "memory");
+}
+
+// 32 consecutive TMEM columns of the warp's 32 lanes
+__device__ __forceinline__ void f4_ld32(uint32_t taddr, uint32_t* d) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+        : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3]), "=r"(d[4]), "=r"(d[5]), "=r"(d[6]), "=r"(d[7]),
+          "=r"(d[8]), "=r"(d[9]), "=r"(d[10]), "=r"(d[11]), "=r"(d[12]), "=r"(d[13]), "=r"(d[14]), "=r"(d[15]),
+          "=r"(d[16]), "=r"(d[17]), "=r"(d[18]), "=r"(d[19]), "=r"(d[20]), "=r"(d[21]), "=r"(d[22]), "=r"(d[23]),
+          "=r"(d[24]), "=r"(d[25]), "=r"(d[26]), "=r"(d[27]), "=r"(d[28]), "=r"(d[29]), "=r"(d[30]), "=r"(d[31])
+        : "r"(taddr)
+        : "memory");
+}
+// an fp32 accumulator holding an integer of magnitude < 2^22 -> that integer (the 1.5 * 2^23 shift)
+__device__ __forceinline__ int f4_int(uint32_t d) {
+    return __float_as_int(__int_as_float((int)d) + 12582912.0f) - 0x4b400000;
 }
 
 // 8 bits -> bit i at bit 4 i
@@ -407,16 +444,21 @@ __global__ void __launch_bounds__(256) fp4_image_kernel(const uint32_t* __restri
     img[(6 + k) * R] = f4_nibbles(va, 0u);
 }
 
+// K2P = false: JC69 keys and line minima (D1, D2); K2P = true: the K2P keys (D1', D2, D3), see above
+template <bool K2P>
 __global__ void __launch_bounds__(TC_THREADS, 1) dense_fp4_kernel(const TcArgs a) {   // a.n_w = chunks of 64 sites
+    constexpr int TN = K2P ? F4K_TN : F4_TN;
+    constexpr int B_BYTES = TN * F4_KS;
+    constexpr int STAGE = F4_A + B_BYTES;
     extern __shared__ unsigned char tc_smem_raw[];
     unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem + F4_STAGES * F4_STAGE);
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + F4_STAGES * STAGE);
     uint64_t* empty = full + F4_STAGES;
     uint64_t* tfull = empty + F4_STAGES;
     uint64_t* tempty = tfull + 1;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 1);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int n_qt = a.q_pad / F4_TM, n_rt = a.r_pad / F4_TN;
+    const int n_qt = a.q_pad / F4_TM, n_rt = a.r_pad / TN;
     const int n_tiles = n_qt * n_rt;
 
     if (tid == 0) {
@@ -461,10 +503,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_fp4_kernel(const TcArgs a
                 for (int c = 0; c < a.n_w; ++c, ++it) {
                     const int s = it % F4_STAGES;
                     tc_mbar_wait(&empty[s], ((it / F4_STAGES) & 1) ^ 1);
-                    tc_mbar_expect_tx(&full[s], F4_STAGE);
-                    unsigned char* sa = smem + (size_t)s * F4_STAGE;
+                    tc_mbar_expect_tx(&full[s], STAGE);
+                    unsigned char* sa = smem + (size_t)s * STAGE;
                     tc_bulk_g2s(sa, a.a_img + ((size_t)qt * a.n_w + c) * F4_A, F4_A, &full[s]);
-                    tc_bulk_g2s(sa + F4_A, a.b_img + ((size_t)rt * a.n_w + c) * F4_B, F4_B, &full[s]);
+                    tc_bulk_g2s(sa + F4_A, a.b_img + ((size_t)rt * a.n_w + c) * B_BYTES, B_BYTES, &full[s]);
                 }
             }
         }
@@ -480,26 +522,71 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_fp4_kernel(const TcArgs a
                     const int s = it % F4_STAGES;
                     tc_mbar_wait(&full[s], (it / F4_STAGES) & 1);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    const uint32_t sa = tc_smem_u32(smem + (size_t)s * F4_STAGE), sb = sa + F4_A;
+                    const uint32_t sa = tc_smem_u32(smem + (size_t)s * STAGE), sb = sa + F4_A;
 #pragma unroll
-                    for (int k = 0; k < 4; ++k) {   // components x, y, z into D1, validity into D2
+                    for (int k = 0; k < 4; ++k) {   // components x, y, z into D1, validity into D2 (K2P: y into D3)
                         const uint64_t ad = tc_desc(sa + 2 * k * (F4_TM * 16), F4_TM * 16, 128);
-                        const uint64_t bd = tc_desc(sb + 2 * k * (F4_TN * 16), F4_TN * 16, 128);
-                        if (k < 3)
-                            f4_mma(tmem, ad, bd, sfa, sfb, (c > 0 || k > 0) ? 1u : 0u);
+                        const uint64_t bd = tc_desc(sb + 2 * k * (TN * 16), TN * 16, 128);
+                        if (K2P && k == 1)
+                            f4_mma<TN>(tmem + F4K_D3, ad, bd, sfa, sfb, c > 0 ? 1u : 0u);
+                        else if (k < 3)
+                            f4_mma<TN>(tmem, ad, bd, sfa, sfb, (c > 0 || k > 0) ? 1u : 0u);
                         else
-                            f4_mma(tmem + F4_D2, ad, bd, sfa, sfb, c > 0 ? 1u : 0u);
+                            f4_mma<TN>(tmem + (K2P ? F4K_D2 : F4_D2), ad, bd, sfa, sfb, c > 0 ? 1u : 0u);
                     }
                     tc_commit(&empty[s]);
                 }
                 tc_commit(tfull);
             }
         }
+    } else if constexpr (K2P) {
+        // ===== K2P epilogue: two warps per TMEM lane quarter; g = 0 takes the lines 0..2 of the tile row, g = 1 the lines 3..4 =====
+        const int quarter = warp & 3, g = (warp - 2) >> 2;
+        const int c0 = g * 96, c1 = g ? F4K_TN : 96;
+        unsigned long long* xp =
+            reinterpret_cast<unsigned long long*>(smem + F4_STAGES * STAGE + 256) + (size_t)(warp - 2) * (F4K_XPOSE / 8);
+        unsigned long long* keys = reinterpret_cast<unsigned long long*>(a.keys);
+        uint32_t tl = 0;
+        for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++tl) {
+            int qt, rt;
+            super_tile(n_qt, n_rt, a.sq, a.sr, t, qt, rt);
+            tc_mbar_wait(tfull, tl & 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const int row0 = qt * F4_TM + quarter * 32;
+#pragma unroll 1
+            for (int c = c0; c < c1; c += 32) {
+                uint32_t d1[32], d2[32], d3[32];
+                const uint32_t taddr = tmem + ((uint32_t)(quarter * 32) << 16) + (uint32_t)c;
+                f4_ld32(taddr, d1);
+                f4_ld32(taddr + F4K_D2, d2);
+                f4_ld32(taddr + F4K_D3, d3);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+                for (int j = 0; j < 32; ++j) {
+                    const int mts2 = f4_int(d1[j]), valid = f4_int(d2[j]), y = f4_int(d3[j]);
+                    const int tv = (valid - y) >> 1;
+                    const int ts = (valid - tv - (mts2 >> 1)) >> 1;
+                    xp[lane * 33 + j] = (unsigned long long)(uint32_t)(ts | (tv << 16)) | ((unsigned long long)valid << 32);
+                }
+                __syncwarp();
+                // 2 rows x 256 bytes per store instruction
+#pragma unroll
+                for (int r0 = 0; r0 < 32; r0 += 2) {
+                    const int rr = r0 + (lane >> 4), cc = (lane & 15) * 2;
+                    const ulonglong2 o = make_ulonglong2(xp[rr * 33 + cc], xp[rr * 33 + cc + 1]);
+                    __stcs(reinterpret_cast<ulonglong2*>(keys + (size_t)(row0 + rr) * a.ldk + (size_t)rt * F4K_TN + c + cc), o);
+                }
+                __syncwarp();
+            }
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            __syncwarp();
+            if (lane == 0) tc_mbar_arrive(tempty);
+        }
     } else {
         // ===== epilogue: two warps per TMEM lane quarter; g = 0 takes the lines 0..3 of the tile row, g = 1 the lines 4..6 =====
         const int quarter = warp & 3, g = (warp - 2) >> 2;
         const int c0 = g * 128, c1 = g ? F4_TN : 128;
-        uint32_t* xp = reinterpret_cast<uint32_t*>(smem + F4_STAGES * F4_STAGE + 256) + (size_t)(warp - 2) * (TC_XPOSE / 4);
+        uint32_t* xp = reinterpret_cast<uint32_t*>(smem + F4_STAGES * STAGE + 256) + (size_t)(warp - 2) * (TC_XPOSE / 4);
         uint32_t tl = 0;
         for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++tl) {
             int qt, rt;
@@ -580,13 +667,15 @@ __global__ void __launch_bounds__(TC_THREADS, 1) dense_fp4_kernel(const TcArgs a
 cudaError_t dense_tc_configure() {
     cudaError_t e = cudaFuncSetAttribute(tc_image_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TCI_SMEM);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(dense_fp4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F4_SMEM);
+    e = cudaFuncSetAttribute(dense_fp4_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, F4_SMEM);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(dense_fp4_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, F4K_SMEM);
     if (e != cudaSuccess) return e;
     return cudaFuncSetAttribute(dense_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
 }
 
 int dense_fp4_max_sites() { return FP4_MAX_L < TC_MAX_L ? FP4_MAX_L : TC_MAX_L; }
-int dense_fp4_tile_rows(int side) { return side ? F4_TN : F4_TM; }
+int dense_fp4_tile_rows(int side, bool k2p) { return side ? (k2p ? F4K_TN : F4_TN) : F4_TM; }
 size_t dense_fp4_image_bytes(int rows_pad, int n_w) { return (size_t)rows_pad * ((n_w + 1) / 2) * F4_KS; }
 
 void launch_fp4_image(const uint32_t* planes, int rows, int W, int n_w, int rows_pad, int tile_rows, void* out, cudaStream_t s) {
@@ -611,7 +700,25 @@ void launch_dense_fp4(const void* a_img, int q_pad, const void* b_img, int r_pad
     a.sq = 12;
     a.sr = 12;
     const int tiles = (q_pad / F4_TM) * (r_pad / F4_TN);
-    dense_fp4_kernel<<<tiles < num_sms ? tiles : num_sms, TC_THREADS, F4_SMEM, s>>>(a);
+    dense_fp4_kernel<false><<<tiles < num_sms ? tiles : num_sms, TC_THREADS, F4_SMEM, s>>>(a);
+}
+
+void launch_dense_fp4_k2p(const void* a_img, int q_pad, const void* b_img, int r_pad, int n_w, unsigned long long* keys,
+                          int64_t ldk, int num_sms, cudaStream_t s) {
+    TcArgs a;
+    a.a_img = (const uint8_t*)a_img;
+    a.b_img = (const uint8_t*)b_img;
+    a.q_pad = q_pad;
+    a.r_pad = r_pad;
+    a.n_w = (n_w + 1) / 2;
+    a.keys = reinterpret_cast<uint32_t*>(keys);
+    a.ldk = ldk;
+    a.kmin = nullptr;
+    a.vmin1 = 1;
+    a.sq = 12;
+    a.sr = 12;
+    const int tiles = (q_pad / F4_TM) * (r_pad / F4K_TN);
+    dense_fp4_kernel<true><<<tiles < num_sms ? tiles : num_sms, TC_THREADS, F4K_SMEM, s>>>(a);
 }
 
 int dense_tc_max_sites() { return TC_MAX_L; }

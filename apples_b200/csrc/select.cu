@@ -60,6 +60,13 @@ struct Key<SEL_MATRIX> {
     double d;
     int idx;
 };
+// SEL_K2P: 64-bit count keys (ts | tv << 16 | valid << 32) of the K2P count kernel, ordered and classified by their K2P
+// distance as SEL_AA is by its fp64 keys
+template <>
+struct Key<SEL_K2P> {
+    double d;
+    int idx;
+};
 
 __device__ __forceinline__ bool key_less(const Key<SEL_NUC>& a, const Key<SEL_NUC>& b) {
     const uint32_t x = a.m * b.v, y = b.m * a.v;  // counts <= 65535: products fit 32 bits
@@ -73,6 +80,9 @@ __device__ __forceinline__ bool key_less(const Key<SEL_AA>& a, const Key<SEL_AA>
     return a.d < b.d || (a.d == b.d && a.idx < b.idx);
 }
 __device__ __forceinline__ bool key_less(const Key<SEL_MATRIX>& a, const Key<SEL_MATRIX>& b) {
+    return a.d < b.d || (a.d == b.d && a.idx < b.idx);
+}
+__device__ __forceinline__ bool key_less(const Key<SEL_K2P>& a, const Key<SEL_K2P>& b) {
     return a.d < b.d || (a.d == b.d && a.idx < b.idx);
 }
 
@@ -151,6 +161,13 @@ template <>
 struct RawT<SEL_NUCW> {
     using T = unsigned long long;   // mismatch | valid << 32
 };
+template <>
+struct RawT<SEL_K2P> {
+    using T = unsigned long long;   // ts | tv << 16 | valid << 32
+};
+__device__ __forceinline__ double k2p_key_dist(unsigned long long raw, int vmin) {
+    return k2p_from_counts((uint32_t)(raw & 0xffffu), (uint32_t)((raw >> 16) & 0xffffu), (uint32_t)(raw >> 32), vmin);
+}
 __device__ __forceinline__ Key<SEL_NUC> make_key_nuc(uint32_t raw, int idx) {
     Key<SEL_NUC> k;
     k.m = raw & 0xffffu;
@@ -175,11 +192,23 @@ __device__ __forceinline__ Key<KIND> make_key(typename RawT<KIND>::T raw, int id
         return k;
     }
 }
+// the generic kernel's keys: K2P keys become their distance (the overlap gate comes from the launch)
+template <int KIND>
+__device__ __forceinline__ Key<KIND> make_key_sel(const SelectArgs& a, typename RawT<KIND>::T raw, int idx) {
+    if constexpr (KIND == SEL_K2P) {
+        Key<SEL_K2P> k;
+        k.d = k2p_key_dist(raw, a.gate.vmin);
+        k.idx = idx;
+        return k;
+    } else {
+        return make_key<KIND>(raw, idx);
+    }
+}
 template <int KIND>
 __device__ __forceinline__ typename RawT<KIND>::T load_raw(const SelectArgs& a, int row, int u) {
     if constexpr (KIND == SEL_NUC)
         return a.keys_nuc[(size_t)row * a.ldk + u];
-    else if constexpr (KIND == SEL_NUCW)
+    else if constexpr (KIND == SEL_NUCW || KIND == SEL_K2P)
         return reinterpret_cast<const unsigned long long*>(a.keys_f64)[(size_t)row * a.ldk + u];
     else
         return a.keys_f64[(size_t)row * a.ldk + u];
@@ -227,6 +256,10 @@ __device__ __forceinline__ int classify(const SelectArgs& a, const Key<SEL_AA>& 
     if (!(k.d >= 0.0)) return 0;  // Reference.py:141
     return k.d <= a.thr ? 1 : 2;
 }
+__device__ __forceinline__ int classify(const SelectArgs& a, const Key<SEL_K2P>& k) {
+    if (!(k.d >= 0.0)) return 0;
+    return k.d <= a.thr ? 1 : 2;
+}
 __device__ __forceinline__ int classify(const SelectArgs& a, const Key<SEL_MATRIX>& k) {
     if (!(k.d >= 0.0) || a.col_node[k.idx] < 0) return 0;  // PoolQueryWorker.py:52
     return k.d <= a.thr ? 1 : 2;
@@ -268,6 +301,49 @@ __device__ __forceinline__ void member_counts_nuc(const SelectArgs& a, const uin
         for (int k = 0; k < NR; ++k) acc[k] += __shfl_xor_sync(FULLMASK, acc[k], o);
 #pragma unroll
     for (int k = 0; k < NR; ++k) out[k] = acc[k];
+}
+
+// K2P twin: (mismatch | valid << 16) as above and the transversions apart (lo differs: purine against pyrimidine)
+template <int NR>
+__device__ __forceinline__ void member_counts_k2p(const SelectArgs& a, const uint32_t* __restrict__ qrow, const int* rows,
+                                                  int lane, uint32_t* out, uint32_t* out_tv) {
+    uint32_t acc[NR], atv[NR];
+#pragma unroll
+    for (int k = 0; k < NR; ++k) acc[k] = atv[k] = 0;
+    for (int w = 4 * lane; w < a.W; w += 128) {
+        const uint4 ql = *reinterpret_cast<const uint4*>(qrow + w);
+        const uint4 qh = *reinterpret_cast<const uint4*>(qrow + a.W + w);
+        const uint4 qv = *reinterpret_cast<const uint4*>(qrow + 2 * a.W + w);
+        uint4 rl[NR], rh[NR], rv[NR];
+#pragma unroll
+        for (int k = 0; k < NR; ++k) {
+            const uint32_t* __restrict__ r = a.refs_nuc + (size_t)rows[k] * 3 * a.W;
+            rl[k] = *reinterpret_cast<const uint4*>(r + w);
+            rh[k] = *reinterpret_cast<const uint4*>(r + a.W + w);
+            rv[k] = *reinterpret_cast<const uint4*>(r + 2 * a.W + w);
+        }
+#pragma unroll
+        for (int k = 0; k < NR; ++k) {
+            uint32_t v, m, d;
+#define APPLES_ACC(c)                                                                                        \
+            v = qv.c & rv[k].c; d = ql.c ^ rl[k].c; m = (d | (qh.c ^ rh[k].c)) & v;                          \
+            acc[k] += __popc(m) + (__popc(v) << 16); atv[k] += __popc(d & v);
+            APPLES_ACC(x) APPLES_ACC(y) APPLES_ACC(z) APPLES_ACC(w)
+#undef APPLES_ACC
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int k = 0; k < NR; ++k) {
+            acc[k] += __shfl_xor_sync(FULLMASK, acc[k], o);
+            atv[k] += __shfl_xor_sync(FULLMASK, atv[k], o);
+        }
+#pragma unroll
+    for (int k = 0; k < NR; ++k) {
+        out[k] = acc[k];
+        out_tv[k] = atv[k];
+    }
 }
 
 // byte-compare twin for the fallback: the reference's own definition on raw bytes (distance.py:733-737): a site counts
@@ -414,6 +490,23 @@ __device__ __forceinline__ void expand_unit(const SelectArgs& a, WarpSel<KIND>& 
 #pragma unroll
                 for (int k = 0; k < NR; ++k)
                     if (x + k < e) observe_nucw_counts(a, st, slot, self, nodes[k], cm[k], cv[k], ukey, x + k - b, lane);
+            }
+        } else if constexpr (KIND == SEL_K2P) {
+            const uint32_t* qrow = a.q_nuc + (size_t)q * 3 * a.W;
+            for (int x = b; x < e && st.kcount <= a.cap; x += NR) {
+                int rows[NR], nodes[NR];
+                uint32_t c[NR], ctv[NR];
+#pragma unroll
+                for (int k = 0; k < NR; ++k) rows[k] = a.gmem[min(x + k, e - 1)];
+#pragma unroll
+                for (int k = 0; k < NR; ++k) nodes[k] = a.ref_node[rows[k]];
+                member_counts_k2p<NR>(a, qrow, rows, lane, c, ctv);
+#pragma unroll
+                for (int k = 0; k < NR; ++k)
+                    if (x + k < e) {
+                        const double d = k2p_from_counts((c[k] & 0xffffu) - ctv[k], ctv[k], c[k] >> 16, a.gate.vmin);
+                        if (!(d < 0.0)) observe<KIND>(a, st, slot, self, nodes[k], d, d == 0.0, ukey, x + k - b, lane);
+                    }
             }
         } else {
             for (int x = b; x < e && st.kcount <= a.cap; ++x) {
@@ -570,6 +663,9 @@ __global__ void __launch_bounds__(32 * SEL_GEN_WARPS, 16 / SEL_GEN_WARPS) select
             if constexpr (KIND == SEL_NUCW) {
                 const uint32_t m = (uint32_t)(raw[j] & 0xffffffffull), v = (uint32_t)(raw[j] >> 32);
                 if ((uint64_t)m * bv < (uint64_t)bm * v) ev |= 1u << j;
+            } else if constexpr (KIND == SEL_K2P) {
+                const int u = u0 + j * 32 + lane;
+                if (u < a.n_units && !(k2p_key_dist(raw[j], a.gate.vmin) > l2.d)) ev |= 1u << j;   // near and missing keys included
             } else {
                 const int u = u0 + j * 32 + lane;
                 if (u < a.n_units && !(raw[j] > l2.d)) ev |= 1u << j;  // NaN and near keys included
@@ -585,7 +681,7 @@ __global__ void __launch_bounds__(32 * SEL_GEN_WARPS, 16 / SEL_GEN_WARPS) select
 #pragma unroll
                 for (int t = 1; t < U; ++t)
                     if (j == t) rj = raw[t];
-                const Key<KIND> kj = make_key<KIND>(rj, u0 + j * 32 + lane);
+                const Key<KIND> kj = make_key_sel<KIND>(a, rj, u0 + j * 32 + lane);
                 const int c = classify(a, kj);
                 if (c == 1) nearb |= 1u << j;
                 if (c == 2 && key_less(kj, l2)) {
@@ -623,7 +719,7 @@ __global__ void __launch_bounds__(32 * SEL_GEN_WARPS, 16 / SEL_GEN_WARPS) select
                     while (nearm[j] && qn < 32) {
                         const int src = __ffs(nearm[j]) - 1;
                         nearm[j] &= nearm[j] - 1;
-                        const Key<KIND> uk = make_key<KIND>(__shfl_sync(FULLMASK, raw[j], src), u0 + j * 32 + src);
+                        const Key<KIND> uk = make_key_sel<KIND>(a, __shfl_sync(FULLMASK, raw[j], src), u0 + j * 32 + src);
                         if (lane == qn) qkey = uk;
                         ++qn;
                     }
@@ -672,7 +768,7 @@ __global__ void __launch_bounds__(32 * SEL_GEN_WARPS, 16 / SEL_GEN_WARPS) select
 #pragma unroll
                 for (int j = 0; j < RU * VEC; ++j) {
                     const int u = ((k0 + 32 * (j / VEC)) * 32 + owner) * VEC + j % VEC;
-                    const Key<KIND> kj = make_key<KIND>(rr[j], u);
+                    const Key<KIND> kj = make_key_sel<KIND>(a, rr[j], u);
                     if (u < a.n_units && classify(a, kj) == 2 && key_less(g, kj) && key_less(kj, n2)) {
                         if (key_less(kj, n1)) {
                             n2 = n1;
@@ -1079,6 +1175,7 @@ void launch_select(int kind, const SelectArgs& a, cudaStream_t s) {
         const dim3 g((a.n + w - 1) / w), b(w * 32);
         if (kind == SEL_NUCW) select_kernel<SEL_NUCW><<<g, b, 0, s>>>(a);
         else if (kind == SEL_AA) select_kernel<SEL_AA><<<g, b, 0, s>>>(a);
+        else if (kind == SEL_K2P) select_kernel<SEL_K2P><<<g, b, 0, s>>>(a);
         else select_kernel<SEL_MATRIX><<<g, b, 0, s>>>(a);
     }
 }

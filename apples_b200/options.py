@@ -4,7 +4,8 @@ apples/OptionsRun.py:5-112 and apples/OptionsBuild.py:4-10, plus two additions t
                     dependency of the reference, Reference.py:87-88)
   --device N        first CUDA device ordinal (default 0); -T/--threads is accepted and ignored (no CPU workers);
   --gpus N          GPUs to shard the queries over (0 = all visible: the analogue of upstream's -T 0 = all cores);
-  --keep-at-most K  report the best K placements of each query (pplacer's name; default 1), ranked by the criterion.
+  --keep-at-most K  report the best K placements of each query (pplacer's name; default 1), ranked by the criterion;
+  --model M         nucleotide distance of alignment input: JC69 (upstream's, default) or K2P (Kimura two-parameter).
 Backbone re-estimation with FastTree (reestimateBackbone.py) is outside the hot path: it is never run here, as with
 the reference's -D flag; without -D a warning says that results can differ from upstream's default.
 """
@@ -82,9 +83,20 @@ def options_config_run(argv=None):
     p.add_option('--keep-at-most', dest='keep_at_most', type=int, default=1, metavar='NUMBER',
                  help='report the best NUMBER (1 to 16) placements of each query in criterion order; the extra ones have '
                       'like_weight_ratio 0')
+    p.add_option('--model', dest='model', default=None, metavar='MODEL',
+                 help='nucleotide distance model of alignment input: JC69 (default) or K2P (Kimura two-parameter)')
     options, args = _parse(p, argv)
     if not 1 <= options.keep_at_most <= 16:
         raise ValueError('--keep-at-most must be from 1 to 16, got %d' % options.keep_at_most)
+    if options.model is not None:
+        if options.model not in ('JC69', 'K2P'):
+            raise ValueError('--model must be JC69 or K2P, got %r' % options.model)
+        if options.protein_seqs:
+            raise ValueError('--model chooses a nucleotide distance; it cannot be combined with -p')
+        if options.dist_fp:
+            raise ValueError('--model applies to alignment input; it cannot be combined with -d')
+    else:
+        options.model = 'JC69'
     # OptionsRun.py:88-110
     if options.dist_fp:
         if options.ref_fp:

@@ -25,7 +25,7 @@ class GpuPlacer:
     """One GPU context holding the replicated read-only state (tree, packed reference, clusters) -- the analogue of
     PoolQueryWorker's fork-inherited class attributes (PoolQueryWorker.py:11-25)."""
 
-    def __init__(self, tree, reference=None, name_to_node_map=None, device=0, matrix_tags=None):
+    def __init__(self, tree, reference=None, name_to_node_map=None, device=0, matrix_tags=None, model='JC69'):
         self.lib = _lib.load()
         self.tree = tree
         self.name_to_node = {k: _edge_index_of(v) for k, v in
@@ -41,6 +41,8 @@ class GpuPlacer:
         import os as _os
         if _os.environ.get('APPLES_B200_DENSE', '') == 'intpipe':
             self._check(self.lib.apples_ctx_set_dense_mode(self.h, 0))
+        self.model = check_model(model)
+        self._check(self.lib.apples_ctx_set_model(self.h, _lib.MODELS[self.model]))
         self._check(self.lib.apples_set_tree(self.h, tree.num_nodes, _lib.ptr(tree.parent), _lib.ptr(tree.edge_length),
                                              _lib.ptr(tree.level), _lib.ptr(tree.first)))
         self.reference = None
@@ -221,13 +223,13 @@ class GpuPlacer:
         return K, V, ov
 
     def timings(self, reset=False):
-        v = np.zeros(24, np.float64)
-        self.lib.apples_get_timings(self.h, _lib.ptr(v), 24, 1 if reset else 0)
+        v = np.zeros(25, np.float64)
+        self.lib.apples_get_timings(self.h, _lib.ptr(v), 25, 1 if reset else 0)
         keys = ['h2d_ms', 'transpose_ms', 'rep_distance_ms', 'selection_ms', 'placement_ms', 'd2h_ms', 'launches',
                 'rep_distance_launches', 'pairs', 'observed', 'valid_nodes', 'overflow_queries', 'max_observed',
                 'max_valid_nodes', 'rep_distance_sm_mhz', 'placed_smem64', 'placed_smem128', 'placed_smem256',
                 'placed_smem512', 'placed_block', 'fallback_queries', 'tensor_core_launches', 'key_lines_read',
-                'fp4_launches']
+                'fp4_launches', 'k2p_launches']
         return dict(zip(keys, v.tolist()))
 
     # ------------------------------------------------------------------------------------------------ parity exports
@@ -243,7 +245,8 @@ class GpuPlacer:
 
     def count_keys(self, packed, params, line_minima=False):
         """Query x representative keys of the hot path's count stage (apples_count_keys): ([nq, n_rep] array, kind) with
-        kind 0 = uint32 mismatch | valid << 16, 1 = uint64 mismatch | valid << 32 (byte mode), 2 = float64 scoredist.
+        kind 0 = uint32 mismatch | valid << 16, 1 = uint64 mismatch | valid << 32 (byte mode), 2 = float64 scoredist,
+        3 = uint64 transitions | transversions << 16 | valid << 32 (model K2P).
         line_minima=True appends the [nq, ceil(n_rep / 32)] uint32 line minima (None unless kind is 0)."""
         packed = np.ascontiguousarray(packed)
         nq = int(packed.shape[0])
@@ -252,7 +255,7 @@ class GpuPlacer:
         kind = _lib.C.c_int32(-1)
         self._check(self.lib.apples_count_keys(self.h, nq, _lib.ptr(packed), _lib.C.byref(params), _lib.C.byref(kind),
                                                _lib.ptr(raw), _lib.ptr(mins) if line_minima else None))
-        dtype = {0: np.uint32, 1: np.uint64, 2: np.float64}[kind.value]
+        dtype = {0: np.uint32, 1: np.uint64, 2: np.float64, 3: np.uint64}[kind.value]
         keys = raw.view(dtype)[:nq * self.n_rep].reshape(nq, self.n_rep)
         if line_minima:
             return keys, kind.value, (mins if kind.value == 0 else None)
@@ -351,6 +354,22 @@ def results_to_jplace(names, in_backbone, out, exclude_intplace=False, log=True,
     return results
 
 
+def check_model(model):
+    """--model: the nucleotide distance, 'JC69' (upstream's, default) or 'K2P' (Kimura two-parameter)"""
+    if model not in _lib.MODELS:
+        raise ValueError('--model must be one of %s, got %r' % (', '.join(sorted(_lib.MODELS)), model))
+    return model
+
+
+def options_model(options, placer=None):
+    """the --model of a run's options (JC69 when the options object predates the flag); a caller-owned placer must have
+    been built with it"""
+    model = check_model(getattr(options, 'model', None) or 'JC69')
+    if placer is not None and placer.model != model:
+        raise ValueError('the options ask for --model %s, the placer was built for %s' % (model, placer.model))
+    return model
+
+
 def check_keep(keep):
     """--keep-at-most K: 1 <= K <= 16 (APPLES_MAX_KEEP)"""
     if isinstance(keep, bool) or int(keep) != keep or not 1 <= keep <= _lib.MAX_KEEP:
@@ -366,7 +385,7 @@ class MultiGpuPlacer:
     analogue of upstream's `mp.Pool(num_thread)` (run_apples.py:101-102); under torchrun the same split runs with one
     process per GPU and a final NCCL gather (apples_b200.parallel)."""
 
-    def __init__(self, tree, reference=None, name_to_node_map=None, devices=(0,), matrix_tags=None):
+    def __init__(self, tree, reference=None, name_to_node_map=None, devices=(0,), matrix_tags=None, model='JC69'):
         from concurrent.futures import ThreadPoolExecutor
         self.devices = [int(d) for d in devices]
         if not self.devices:
@@ -374,9 +393,11 @@ class MultiGpuPlacer:
         self.pool = ThreadPoolExecutor(max_workers=len(self.devices))
         # contexts are built in parallel: each uploads its own replica of the reference
         self.placers = list(self.pool.map(
-            lambda d: GpuPlacer(tree, reference, name_to_node_map, device=d, matrix_tags=matrix_tags), self.devices))
+            lambda d: GpuPlacer(tree, reference, name_to_node_map, device=d, matrix_tags=matrix_tags, model=model),
+            self.devices))
         p0 = self.placers[0]
         self.name_to_node, self.L, self.kind, self.ref_names = p0.name_to_node, p0.L, p0.kind, p0.ref_names
+        self.model = p0.model
         self.matrix_tags = p0.matrix_tags
         self.params_from_options = p0.params_from_options
 
@@ -469,10 +490,11 @@ def place_arrays(reference, options, name_to_node_map, queries, tree=None, place
             raise ValueError('place_batch needs the BackboneTree (tree=) or a GpuPlacer (placer=)')
         devs = [int(d) for d in devices] if devices else [int(device)]
         devs = devs[:max(1, min(len(devs), hi - lo))]
+        model = options_model(options)
         if len(devs) > 1:
-            placer = MultiGpuPlacer(tree, reference, name_to_node_map, devices=devs)
+            placer = MultiGpuPlacer(tree, reference, name_to_node_map, devices=devs, model=model)
         else:
-            placer = GpuPlacer(tree, reference, name_to_node_map, device=devs[0])
+            placer = GpuPlacer(tree, reference, name_to_node_map, device=devs[0], model=model)
     try:
         t_before = placer.timings()
         in_backbone = [n in placer.name_to_node for n in names]
@@ -505,6 +527,7 @@ def place_arrays(reference, options, name_to_node_map, queries, tree=None, place
                         rows[i, col[t]] = v
             res = placer.place_rows(rows, self_node, params, keep=keep) if mine else _empty_outputs(placer, keep)
         else:
+            options_model(options, placer)
             params = placer.params_from_options(options, reference)
             mat = _fasta.as_byte_matrix([q[1] for q in mine], placer.L)
             res = placer.place_bytes(mat, self_node, params, keep=keep) if mine else _empty_outputs(placer, keep)
@@ -579,10 +602,11 @@ def place_alignment(reference, options, name_to_node_map, names, mat, tree=None,
             raise ValueError('place_alignment needs the BackboneTree (tree=) or a GpuPlacer (placer=)')
         devs = [int(d) for d in devices] if devices else [int(device)]
         devs = devs[:max(1, min(len(devs), hi - lo))]
+        model = options_model(options)
         if len(devs) > 1:
-            placer = MultiGpuPlacer(tree, reference, name_to_node_map, devices=devs)
+            placer = MultiGpuPlacer(tree, reference, name_to_node_map, devices=devs, model=model)
         else:
-            placer = GpuPlacer(tree, reference, name_to_node_map, device=devs[0])
+            placer = GpuPlacer(tree, reference, name_to_node_map, device=devs[0], model=model)
     try:
         t_before = placer.timings()
         n2n = placer.name_to_node
@@ -590,6 +614,7 @@ def place_alignment(reference, options, name_to_node_map, names, mat, tree=None,
         self_node = np.full(hi - lo, -1, np.int32)
         for i in np.flatnonzero(in_backbone[lo:hi]).tolist():
             self_node[i] = n2n[names[lo + i]]
+        options_model(options, placer)
         params = placer.params_from_options(options, reference)
         if mat.shape[1] != placer.L:
             raise ValueError('query alignment has %d columns, reference has %d' % (mat.shape[1], placer.L))

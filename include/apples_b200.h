@@ -88,6 +88,18 @@ int apples_ctx_set_limits(apples_ctx* ctx, int64_t max_subbatch, int64_t scratch
  * integer-pipe kernel automatically. */
 int apples_ctx_set_dense_mode(apples_ctx* ctx, int32_t mode);
 
+/* Substitution model of the nucleotide distances of alignment input.  APPLES_JC69 (default) is upstream's Jukes-Cantor
+ * distance.  APPLES_K2P is the Kimura two-parameter distance: with P and Q the fractions of transitions (A<->G, C<->T) and
+ * transversions among the valid sites (overlap gate as for JC69),
+ *     d = -0.5 ln(1 - 2P - Q) - 0.25 ln(1 - 2Q),   missing when 1 - 2P - Q <= 0 or 1 - 2Q <= 0,   0 without differences.
+ * The representatives, the two-phase selection and the placement are upstream's, with K2P in place of JC69.  Call before
+ * apples_set_reference*: the model fixes the representative image and the key width.  apples_set_reference* fail for a
+ * K2P context with APPLES_AA, with dense mode 0, with more than 33 816 columns, or with reference bytes other than
+ * A,C,G,T,-; a place call fails on the first query row holding such bytes.  Distance-matrix calls ignore the model. */
+#define APPLES_JC69 0
+#define APPLES_K2P 1
+int apples_ctx_set_model(apples_ctx* ctx, int32_t model);
+
 /* Backbone tree as flat arrays over the M nodes (replaces the treeswift node graph prepared by
  * prepareTree.py:24-34 + util.py:57-88).  parent[root] = -1; edge_length of a node is the length of the edge above
  * it; level = BFS depth (root 0); first[u] = smallest id in the subtree of u. */
@@ -167,6 +179,7 @@ int apples_distance_counts(apples_ctx* ctx, int64_t nq, const void* packed_queri
  *   0  uint32  mismatch | valid << 16   (tensor-core or integer-pipe kernel)
  *   1  uint64  mismatch | valid << 32   (byte-compare fallback: L > 65 535 or bytes other than A,C,G,T,- in the reference)
  *   2  double  scoredist with params->overlap_frac (APPLES_AA)
+ *   3  uint64  transitions | transversions << 16 | valid << 32   (APPLES_K2P contexts)
  * The caller sizes keys for 8 bytes per entry unless it knows the context's kind.
  * line_minima (optional, NULL = not wanted; written for kind 0 only) is [nq][ceil(n_rep / 32)]: per line of 32 keys
  * [32 l, 32 l + 32), the key of smallest ratio mismatch / valid among the keys with valid >= max(vmin, 1) and
@@ -201,7 +214,8 @@ int apples_last_counts(apples_ctx* ctx, int64_t n, int32_t* K, int32_t* V, int32
  * block-per-query launch (global scratch)  [20] queries that went through the byte-compare fallback
  * [21] representative-distance launches that ran on the tensor cores
  * [22] key lines (32 keys) the nucleotide selection opened, first pass
- * [23] representative-distance launches that ran the block-scaled fp4 tensor-core kernel (counted in [21] too) */
+ * [23] representative-distance launches that ran the block-scaled fp4 tensor-core kernel (counted in [21] too)
+ * [24] representative-distance launches that ran its K2P instantiation (counted in [21] and [23] too) */
 int apples_get_timings(apples_ctx* ctx, double* out, int n, int reset);
 
 /* ---- host side of SURVEY.md section 8 (f1) / (f3) in native code (no CUDA kernel involved) ---- */
